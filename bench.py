@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR
 
 Metric (BASELINE.json): secp256k1 MSM throughput in Mpts/s at 2^20 points per GPU; a "step" is one
 full multi-scalar multiplication over the resident 2^20-term slice (N > 1: slice MSM on every
@@ -14,6 +15,7 @@ launcher-side rendezvous for N > 1 (NCCL id exchange, barriers, max-over-ranks o
 The oracle (oracle/) is used here only for the cpu_baseline leg and for the in-bench parity check.
 """
 import argparse
+import atexit
 import ctypes
 import json
 import os
@@ -26,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the bench writes nothing into the source tree (it may be read-only): no __pycache__
 # the batch verifier's OpenMP workers must sleep, not spin, between chunks: with one process per GPU on a shared host the spinning
 # pools starve each other (read by libgomp when it is loaded, so it has to be set before any import that pulls it in)
 os.environ.setdefault("OMP_WAIT_POLICY", "PASSIVE")
@@ -61,6 +64,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(index), "--query-gpu=" + self.Q,
                                           "--format=csv,noheader,nounits", "-lms", "200"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)      # a bench that fails before stop() must not leave nvidia-smi sampling behind
             threading.Thread(target=self._pump, daemon=True).start()
         except OSError:
             self.proc = None
@@ -130,6 +134,7 @@ def run_ref_runner(argv, timeout=900):
     env = dict(os.environ)
     for k in ("OMP_NUM_THREADS", "MKL_NUM_THREADS"):     # torchrun pins these to 1; the CPU arm uses every host core
         env.pop(k, None)
+    env["PYTHONDONTWRITEBYTECODE"] = "1"
     try:
         out = subprocess.run([sys.executable, "-m", "oracle.ref_runner"] + argv, cwd=ROOT, env=env, capture_output=True, text=True, timeout=timeout)
     except subprocess.TimeoutExpired:
@@ -340,19 +345,36 @@ def run_ours(args):
         line["bit_exact_vs_oracle"] = bit_exact
     if sharded_ok is not None:
         line["sharded_result_equals_sum_of_slices"] = sharded_ok
+    accept = None
     if not args.no_verify:
         try:
-            line["verify"] = bench_verify(args, nat, dist, rank, world, peak)
+            line["verify"], accept = bench_verify(args, nat, dist, rank, world, peak)
         except Exception as e:   # noqa: BLE001  -- the headline metric must still print
             import traceback
             line["verify"] = {"error": repr(e), "trace": traceback.format_exc()[-600:]}
     lib.bp_handle_free(hp)
     lib.bp_handle_free(hs)
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, result_hex, accept)
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(dirname, result_hex, accept):
+    """What the timed paths handed their caller in their last step, as arrays on which two builds can be compared:
+      msm_result.npy     (2, 8) float64: x and y of the affine MSM result as 32-bit little-endian limbs (exact in float64);
+                         the identity is all zero
+      verify_accept.npy  (proofs,) float32: the decisions of the last timed batch verification, 1 = accepted, 0 = rejected
+                         (absent with --no-verify or when the verify leg failed)"""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    limbs = np.frombuffer(bytes.fromhex(result_hex), dtype="<u4").astype(np.float64).reshape(2, 8)
+    np.save(os.path.join(dirname, "msm_result.npy"), limbs)
+    if accept is not None:
+        np.save(os.path.join(dirname, "verify_accept.npy"), np.frombuffer(accept, dtype=np.uint8).astype(np.float32))
 
 
 def measured_hbm():
@@ -561,7 +583,7 @@ def bench_verify(args, nat, dist, rank, world, imad_peak):
                 res["aggregated"] = bench_verify_aggregated(nat, q)
             except Exception as e:   # noqa: BLE001
                 res["aggregated"] = {"error": repr(e)}
-    return res
+    return res, acc
 
 
 def bench_verify_aggregated(nat, q, m=16, nbits=64, distinct=32, total=2048):
@@ -730,7 +752,13 @@ def main():
     ap.add_argument("--verify-prover-check", type=int, default=16)
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--no-precompute", action="store_true", help="time the plain bucket method as the headline (no per-vector precomputation)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the outputs of the last step as DIR/<name>.npy "
+                    "(same arguments, same inputs: two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
