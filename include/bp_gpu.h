@@ -56,13 +56,8 @@ int bp_handle_free(bp_handle h);
 int bp_points_precompute(bp_handle points, int window_bits);
 int bp_points_pre_info(bp_handle points, int* window_bits, int* windows, uint64_t* bytes);
 int bp_msm_set_small_graphs(int on);      /* MSMs of <= 2^17 terms over a precomputed vector as replayed CUDA graphs (default on) */
-int bp_msm_set_affine_passes(int passes); /* batched-affine pair passes ahead of the XYZZ accumulation on that path: experiment switch, <= 0 = off (default): measured slower at 2^20, see DESIGN.md 5 */
-int bp_msm_set_chunk_fit(int on);       /* experiment switch: 1 = entries per accumulation thread fitted to whole waves of resident threads, 0 (default; measured no gain) = the fixed 8 / 16 / 32 */
-int bp_msm_set_tails2d(int on);         /* experiment switch: 1 = 2-D marginal bucket reduction for the wide units of a large plain MSM, 0 (default; measured faster) = running sums */
-int bp_msm_set_pre_fused(int on);       /* experiment switch: 1 (default) = the scatter pass of the precomputed path recomputes the digits, 0 = digit array in between */
 int bp_msm_set_pre_slots(int mode, size_t min_terms);   /* sort stage of one large resident MSM (precomputed path; plain path where a bucket holds >= 48 entries, i.e. from 2^20 terms): 1 (default) = slot sort (one scattered pass; exact counting sort as gated fallback) for MSMs of >= min_terms terms (default 2^18; 0 keeps the value), 0 = exact counting sort only, 2 = test hook, 8 slots per bucket so that the fallback runs */
 int bp_msm_set_host_finish(int on);     /* 1 (default): an MSM whose result goes to the host (bp_msm, bp_msm_sharded_host on one rank; bucket method without precomputed multiples) hands its window sums to the host, which runs the Horner chain and the affine conversion; 0 = k_combine on the device */
-int bp_msm_set_pre_chunk(int entries);   /* experiment switch: entries per accumulation thread on that path (0 = automatic) */
 int bp_msm_h(bp_handle points, const uint8_t* sc32, size_t n, uint8_t out64[64]);     /* scalars from host */
 int bp_msm_hh(bp_handle points, bp_handle scalars, size_t n, uint8_t out64[64]);      /* all resident */
 /* XYZZ partial (4 x 32-byte LE: X, Y, ZZ, ZZZ) of a point slice, for sharding over GPUs
@@ -85,8 +80,6 @@ int bp_msm_set_profiling(int on);
 /* kernels this library has launched so far in this process (kernel nodes of a replayed CUDA graph count at every replay);
  * bench.py reports the difference across its timed region as "gpu_launches" */
 int bp_launch_count(uint64_t* launches);
-/* single MSMs with at least this many terms run with their windows pipelined over streams (0 = never) */
-int bp_msm_set_pipeline_min(size_t min_terms);
 int bp_msm_stage_ms(float out7[7]);
 int bp_msm_accumulate_kernel_ms(float* ms);   /* k_accumulate alone (stage [3] also holds the bucket memset and the fix-ups) */
 

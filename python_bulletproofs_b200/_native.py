@@ -29,13 +29,8 @@ PROTOTYPES = {
     "bp_scalars_upload": (ctypes.c_int, [c_u8p, c_sz, ctypes.POINTER(c_h)]),
     "bp_handle_free": (ctypes.c_int, [c_h]),
     "bp_points_precompute": (ctypes.c_int, [c_h, ctypes.c_int]),
-    "bp_msm_set_chunk_fit": (ctypes.c_int, [ctypes.c_int]),
-    "bp_msm_set_tails2d": (ctypes.c_int, [ctypes.c_int]),
-    "bp_msm_set_pre_fused": (ctypes.c_int, [ctypes.c_int]),
     "bp_msm_set_pre_slots": (ctypes.c_int, [ctypes.c_int, c_sz]),
     "bp_msm_set_host_finish": (ctypes.c_int, [ctypes.c_int]),
-    "bp_msm_set_pre_chunk": (ctypes.c_int, [ctypes.c_int]),
-    "bp_msm_set_affine_passes": (ctypes.c_int, [ctypes.c_int]),
     "bp_msm_set_small_graphs": (ctypes.c_int, [ctypes.c_int]),
     "bp_points_pre_info": (ctypes.c_int, [c_h, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_uint64)]),
     "bp_msm_h": (ctypes.c_int, [c_h, c_u8p, c_sz, c_u8p]),
@@ -48,7 +43,6 @@ PROTOTYPES = {
     "bp_msm_last_entries": (ctypes.c_int, [ctypes.POINTER(ctypes.c_uint64)]),
     "bp_msm_set_profiling": (ctypes.c_int, [ctypes.c_int]),
     "bp_launch_count": (ctypes.c_int, [ctypes.POINTER(ctypes.c_uint64)]),
-    "bp_msm_set_pipeline_min": (ctypes.c_int, [c_sz]),
     "bp_msm_stage_ms": (ctypes.c_int, [ctypes.POINTER(ctypes.c_float)]),
     "bp_msm_accumulate_kernel_ms": (ctypes.c_int, [ctypes.POINTER(ctypes.c_float)]),
     "bp_scalar_mul_batch": (ctypes.c_int, [c_u8p, c_u8p, c_sz, c_u8p]),

@@ -40,10 +40,8 @@ int fail(const char* fmt, ...) {
 static int msm_tails(const XYZZ* buckets, const MsmShape& sh, u32 nmsm, Affine* out_affine, XYZZ* out_xyzz, bool prof, cudaStream_t st) {
   const size_t nmw = (size_t)nmsm * sh.U;
   const bool plain_tails = nmsm >= 2048 && sh.H <= 512;     // big batch of small MSMs: throughput forms
-  const bool tails2d = !plain_tails && sh.seg_plain && sh.H >= 4096 && g.tails2d;
-  const size_t nb_all = nmw * sh.H;
-  XYZZ* segsum = (XYZZ*)g.ws_segsum.ensure((tails2d ? nb_all / 4 + 4096 : nmw * sh.nseg) * sizeof(XYZZ));
-  XYZZ* winsum = (XYZZ*)g.ws_winsum.ensure((tails2d ? 2 : 1) * nmw * sizeof(XYZZ));
+  XYZZ* segsum = (XYZZ*)g.ws_segsum.ensure(nmw * sh.nseg * sizeof(XYZZ));
+  XYZZ* winsum = (XYZZ*)g.ws_winsum.ensure(nmw * sizeof(XYZZ));
   if (!segsum || !winsum) return fail("workspace allocation failed");
   size_t nsegs = nmw * sh.nseg;
   const XYZZ* ws;
@@ -55,29 +53,6 @@ static int msm_tails(const XYZZ* buckets, const MsmShape& sh, u32 nmsm, Affine* 
     // ~126 doublings is pure latency and the 4-lane form (2.3 -> 1.3 us per doubling) wins
     if (nmsm <= 12288 && !out_affine) ++g.nlaunch, k_combine<<<(unsigned)((4 * (size_t)nmsm + 127) / 128), 128, 0, st>>>(ws, sh, nmsm, out_affine, out_xyzz);
     else ++g.nlaunch, k_combine_plain<<<(unsigned)((nmsm + 127) / 128), 128, 0, st>>>(ws, sh, nmsm, out_affine, out_xyzz);
-  } else if (tails2d) {
-    // wide units (a large single MSM at c = 16: 9 units of 2^15 buckets): the 2-D marginal reduction of the pre path, all units
-    // side by side -- plain sums of independent thread-level additions down to R + C marginals per unit, only those take a
-    // (<= 9-bit) weight.  Unit u's window sum leaves k_pre_total as two addends; k_combine (pair mode) adds them in its Horner pass.
-    // Parity-green, measured on B200 and left OFF (gpurun_out/tails2d.log): reduce stage 0.300 -> 0.452 ms at 2^20 (2^17: 0.308 ->
-    // 0.450), e2e 2^20 3.48 -> 3.66 ms.  What is a latency chain for ONE unit (pre path: 0.06 + 0.13 ms) turns throughput bound
-    // for nine: 3456 weighted-marginal blocks of 16 quads are three waves of the 4-lane cooperative form, which pays ~2.4x the
-    // multiplications' issue cost in glue; the running-sum levels below do 2 additions per bucket in thread-level form instead.
-    const int lgH = sh.c - 1, lgC = (lgH + 1) / 2, lgR = lgH - lgC;
-    const u32 C = 1u << lgC, R = 1u << lgR;
-    const size_t nb = nb_all;
-    XYZZ* ping = segsum; XYZZ* two = winsum;
-    XYZZ* wsum = (XYZZ*)g.ws_grpsum.ensure(nmw * (size_t)(C + R) * sizeof(XYZZ));
-    if (!wsum) return fail("workspace allocation failed");
-    const u32 Kr = 8, Kc = 8, np_r = C / Kr, np_c = R / Kc;
-    XYZZ* rpart = ping; XYZZ* cpart = ping + (nb / 8 + 2048);
-    const u32 nrow_out = R * np_r, ncol_out = np_c * C;
-    ++g.nlaunch, k_pre_marginals<<<dim3(((nrow_out > ncol_out ? nrow_out : ncol_out) + 127) / 128, 2, (unsigned)nmw), 128, 0, st>>>(
-        buckets, rpart, nrow_out, Kr, buckets, cpart, np_c, C, Kc, sh.H);
-    ++g.nlaunch, k_pre_rowcol<<<dim3(C + R, (unsigned)nmw), 64, 0, st>>>(rpart, np_r, cpart, np_c, C, R, wsum, (u32)sh.U, sh.dbl);
-    ++g.nlaunch, k_pre_total<<<dim3(2, (unsigned)nmw), 256, 0, st>>>(wsum, C, R, two, lgC);
-    if (prof) cudaEventRecord(g.ev[5], st);
-    ++g.nlaunch, k_combine<<<(unsigned)((4 * (size_t)nmsm + 127) / 128), 128, 0, st>>>(two, sh, nmsm, out_affine, out_xyzz, 1);
   } else {
     XYZZ* seg_run = (XYZZ*)g.ws_segrun.ensure(nsegs * sizeof(XYZZ));
     if (!seg_run) return fail("workspace allocation failed");
@@ -118,14 +93,13 @@ static int msm_tails(const XYZZ* buckets, const MsmShape& sh, u32 nmsm, Affine* 
 
 // ---- the MSM pipeline on device-resident operands ----------------------------------------------
 // points/point_idx/scalars/offsets are device pointers; out_affine/out_xyzz device (either may be null)
-static int msm_run_pipelined(const Affine* points, const u32* point_idx, const Fq* scalars, u32 T, Affine* out_affine, XYZZ* out_xyzz);
 // Per-call options of msm_run (passed by value: nothing a failed call could leave behind for the next one).
 //   skip_below  terms whose point index is below this count as zero scalars (the caller evaluates them elsewhere, see k_digits)
 //   pts_ready   event the points are complete at (host-operand MSM whose points upload on the copy stream)
-//   halves      the points arrive in `parts` equal parts (g.ev_half[0 .. parts-1], upload_operands);
-//   split_sort  ... each behind its own scalars (g.ev_part_sc[k]): sort part by part (msm_run_parts)
+//   parts       0, or the operands arrive in that many parts, each its scalars (g.ev_part_sc[k]) followed by its points
+//               (g.ev_half[k]; upload_operands): sorted and accumulated part by part (msm_run_parts)
 //   host_finish the result goes to the host: leave the window sums for horner_host instead of running k_combine (g.hf)
-struct MsmOpts { u32 skip_below = 0; cudaEvent_t pts_ready = nullptr; bool halves = false; int parts = 0; bool split_sort = false; bool host_finish = false; };
+struct MsmOpts { u32 skip_below = 0; cudaEvent_t pts_ready = nullptr; int parts = 0; bool host_finish = false; };
 // Host-operand MSM whose operands arrive in K parts, each part = its scalars followed by its points (upload_operands): every part
 // is sorted on its own as soon as its scalars are in (digits, scan, scatter over T/K terms) and accumulated as soon as its points
 // are in, all parts adding into ONE bucket set (k_accumulate's `into`); reduction and combination are those of a single MSM.
@@ -206,32 +180,16 @@ struct HfScope { HfScope(bool want) { g.hf_want = want && g.hf_enabled; g.hf.pen
 int msm_run(const Affine* points, const u32* point_idx, const Fq* scalars, u32 T, const u32* d_offsets, u32 nmsm,
             size_t terms_per_msm, Affine* out_affine, XYZZ* out_xyzz, MsmOpts opt = MsmOpts()) {
   HfScope hf_scope(opt.host_finish && nmsm == 1 && !g.profiling);
-  if (nmsm == 1 && T >= g.pipeline_min_terms && !g.profiling) {
-    if (opt.pts_ready) BP_CUDA(cudaStreamWaitEvent(g.stream, opt.pts_ready, 0));
-    if (opt.halves) BP_CUDA(cudaStreamWaitEvent(g.stream, g.ev_half[opt.parts - 1], 0));
-    return msm_run_pipelined(points, point_idx, scalars, T, out_affine, out_xyzz);
+  if (opt.parts) {
+    if (nmsm != 1 || point_idx || d_offsets || T < 64 || opt.parts < 2 || opt.parts > 8)
+      return fail("msm: operands in %d parts need one MSM of >= 64 terms without index or offset lists", opt.parts);
+    return msm_run_parts(points, scalars, T, (u32)opt.parts, out_affine, out_xyzz);
   }
   cudaStream_t st = g.stream;
-  // host-operand MSM whose points are still arriving in K parts (upload_operands): ONE digit/sort pass with the part as the major
-  // sort key -- bucket ids (part, unit, digit) -- then one accumulation per part as it lands, all parts adding into the SAME
-  // bucket values (k_accumulate's `into`), so the reduction and combination are those of a single MSM
-  if (opt.halves && opt.split_sort && nmsm == 1 && !point_idx && !d_offsets && T >= 64 && opt.parts >= 2 && opt.parts <= 8)
-    return msm_run_parts(points, scalars, T, (u32)opt.parts, out_affine, out_xyzz);
-  const bool halves = opt.halves && nmsm == 1 && !point_idx && !d_offsets && T >= 64 && opt.parts >= 2 && opt.parts <= 8;
-  if (opt.halves && !halves) BP_CUDA(cudaStreamWaitEvent(st, g.ev_half[opt.parts - 1], 0));      // (cannot happen today: such MSMs have >= 2^17 terms)
-  const u32 K = halves ? (u32)opt.parts : 1;
-  u32 h_ho[9];
-  for (u32 k = 0; k <= K; k++) h_ho[k] = (u32)((unsigned long long)T * k / K);      // part k = terms [h_ho[k], h_ho[k+1])
-  if (halves) {
-    u32* d_ho = (u32*)g.ws_halfoff.ensure(16 * sizeof(u32));
-    if (!d_ho) return fail("workspace allocation failed");
-    BP_CUDA(cudaMemcpyAsync(d_ho, h_ho, (K + 1) * sizeof(u32), cudaMemcpyHostToDevice, st));    // (pageable copy: staged by the driver)
-    d_offsets = d_ho; nmsm = K; terms_per_msm = (T + K - 1) / K;
-  }
   MsmShape sh = msm_shape(terms_per_msm, nmsm, g.force_c);
   g.last_c = sh.c;
-  g.last_nb = (size_t)(halves ? 1 : nmsm) * sh.U * sh.H;
-  size_t nmw = (size_t)nmsm * sh.U, nb = nmw * sh.H;      // bucket ids of the sort (K parts: K * hb)
+  size_t nmw = (size_t)nmsm * sh.U, nb = nmw * sh.H;
+  g.last_nb = nb;
   bool prof = g.profiling;
   if (prof) for (int i = 0; i < 7; i++) cudaEventRecord(g.ev[i], st), (void)0;
   if (T == 0) {   // all identities
@@ -249,14 +207,12 @@ int msm_run(const Affine* points, const u32* point_idx, const Fq* scalars, u32 T
   u32* cursor = (u32*)g.ws_cursor.ensure((nb + 1) * sizeof(u32));
   size_t ntiles = (nb + 1 + BP_SCAN_TILE - 1) / BP_SCAN_TILE;
   u32* tiles = (u32*)g.ws_tiles.ensure(ntiles * sizeof(u32));
-  const size_t nbv = halves ? nb / K : nb;                  // bucket VALUES (the K parts share one set)
-  XYZZ* buckets = (XYZZ*)g.ws_buckets.ensure(nbv * sizeof(XYZZ));
+  XYZZ* buckets = (XYZZ*)g.ws_buckets.ensure(nb * sizeof(XYZZ));
   XYZZ* segsum = (XYZZ*)g.ws_segsum.ensure(nmw * sh.nseg * sizeof(XYZZ));
   XYZZ* winsum = (XYZZ*)g.ws_winsum.ensure(nmw * sizeof(XYZZ));
   // every (term, window) pair is at most one entry, so E <= W*T: size the chunk structures for the bound
   size_t emax = (size_t)sh.W * 2 * T, nchunks = (emax + sh.chunk - 1) / sh.chunk;
-  const size_t hchunks = ((size_t)sh.W * 2 * ((T + K - 1) / K + 1) + sh.chunk - 1) / sh.chunk + 1;      // per part
-  XYZZ* part = (XYZZ*)g.ws_part.ensure(2 * (halves ? K * hchunks : nchunks) * sizeof(XYZZ));
+  XYZZ* part = (XYZZ*)g.ws_part.ensure(2 * nchunks * sizeof(XYZZ));
   const u32 big_cap = (u32)(emax / ((size_t)sh.chunk * (BP_FIXUP_SERIAL_MAX - 1)) + 16);      // buckets that can span that many chunks
   u32* big = (u32*)g.ws_big.ensure((2 * (size_t)big_cap + 4) * sizeof(u32));
   u32* zero_word = big + 2 * (size_t)big_cap + 3;
@@ -267,7 +223,7 @@ int msm_run(const Affine* points, const u32* point_idx, const Fq* scalars, u32 T
   // (only where a bucket holds >= 48 entries: at a bucket boundary k_accumulate_slots fetches the next entry AFTER the flush, an
   //  exposed load per boundary -- 2^18 terms, 16 entries per bucket: accumulate 0.567 -> 0.624 ms, the whole MSM 1.19 -> 1.23 ms;
   //  2^20 terms, 64 per bucket: 2.870 -> 2.798 ms.  Mode 2, the test hook, takes every size.)
-  const bool use_slots = g.pre_slots > 0 && nmsm == 1 && !halves && !d_offsets && !point_idx && !opt.skip_below && T >= g.pre_slots_min &&
+  const bool use_slots = g.pre_slots > 0 && nmsm == 1 && !d_offsets && !point_idx && !opt.skip_below && T >= g.pre_slots_min &&
                          (g.pre_slots == 2 || 2.0 * (double)T / (double)sh.H >= 48.0 || g.pre_slots_any);
   u32 cap = 0; u32* slots = nullptr; u32* overflow = nullptr;
   if (use_slots) {
@@ -293,131 +249,22 @@ int msm_run(const Affine* points, const u32* point_idx, const Fq* scalars, u32 T
   ++g.nlaunch, k_scatter<<<(2 * T + 255) / 256, 256, 0, st>>>(digits, T, d_offsets, nmsm, sh, cursor, entries, overflow);
   if (prof) cudaEventRecord(g.ev[3], st);
   g.dbg_rec(5, st);
-  BP_CUDA(cudaMemsetAsync(buckets, 0, nbv * sizeof(XYZZ), st));         // empty buckets = identity (ZZ = 0)
+  BP_CUDA(cudaMemsetAsync(buckets, 0, nb * sizeof(XYZZ), st));          // empty buckets = identity (ZZ = 0)
   BP_CUDA(cudaMemsetAsync(zero_word, 0, sizeof(u32), st));
   BP_CUDA(cudaMemsetAsync(big, 0, 2 * sizeof(u32), st));   // [0] = queue length, kept zero word for gs = 0 lives at big[big_cap + 1]
-  if (halves) {
-    const size_t hb = (size_t)sh.U * sh.H;                  // buckets of one part; entries of part k are [start[k*hb], start[(k+1)*hb])
-    for (u32 k = 0; k < K; k++) {
-      const u32 t0 = h_ho[k], tn = h_ho[k + 1] - h_ho[k];
-      BP_CUDA(cudaStreamWaitEvent(st, g.ev_half[k], 0));    // this part of the points has landed
-      ++g.nlaunch, k_phi<<<(tn + 127) / 128, 128, 0, st>>>(points + t0, nullptr, tn, phi + t0);
-      const u32* gs = k ? start + k * hb : zero_word;
-      XYZZ* part_k = part + 2 * (size_t)k * hchunks;
-      if (prof && k == 0) cudaEventRecord(g.ev_k0, st);
-      ++g.nlaunch, k_accumulate<<<(unsigned)((hchunks + 127) / 128), 128, 0, st>>>(points, nullptr, phi, start, entries, gs, start + (k + 1) * hb, sh.chunk, buckets, part_k, (u32)hb, k ? 1 : 0);
-      if (prof && k == K - 1) cudaEventRecord(g.ev_k1, st);
-      if (k) BP_CUDA(cudaMemsetAsync(big, 0, 2 * sizeof(u32), st));
-      ++g.nlaunch, k_fixup<<<(unsigned)((hb + 127) / 128), 128, 0, st>>>(start, k * hb, hb, gs, sh.chunk, part_k, buckets, big, big_cap, (u32)hb);
-      ++g.nlaunch, k_fixup_mid<<<2 * g.sm_count, 256, 0, st>>>(start, gs, sh.chunk, part_k, buckets, big, big_cap, (u32)hb);
-      ++g.nlaunch, k_fixup_big<<<g.sm_count, 256, 0, st>>>(start, gs, sh.chunk, part_k, buckets, big, (u32)hb);
-      g.dbg_rec(6 + (k == K - 1 ? 1 : 0), st);
-    }
-  } else {
-    if (opt.pts_ready) BP_CUDA(cudaStreamWaitEvent(st, opt.pts_ready, 0));   // points may still be uploading
-    ++g.nlaunch, k_phi<<<(T + 127) / 128, 128, 0, st>>>(points, point_idx, T, phi);
-    // E (= start[nb]) stays on the device: launch for the upper bound W*T, threads past E exit at once
-    if (prof) cudaEventRecord(g.ev_k0, st);
-    if (use_slots) ++g.nlaunch, k_accumulate_slots<true><<<(unsigned)((nchunks + 127) / 128), 128, 0, st>>>(points, phi, start, (u32)nb, slots, cap, overflow, sh.chunk, buckets, part);
-    ++g.nlaunch, k_accumulate<<<(unsigned)((nchunks + 127) / 128), 128, 0, st>>>(points, point_idx, phi, start, entries, zero_word, start + nb, sh.chunk, buckets, part, 0, 0, overflow);
-    if (prof) cudaEventRecord(g.ev_k1, st);
-    ++g.nlaunch, k_fixup<<<(unsigned)((nb + 127) / 128), 128, 0, st>>>(start, 0, nb, zero_word, sh.chunk, part, buckets, big, big_cap);
-    ++g.nlaunch, k_fixup_mid<<<2 * g.sm_count, 256, 0, st>>>(start, zero_word, sh.chunk, part, buckets, big, big_cap);
-    ++g.nlaunch, k_fixup_big<<<g.sm_count, 256, 0, st>>>(start, zero_word, sh.chunk, part, buckets, big);
-  }
-  if (prof) cudaEventRecord(g.ev[4], st);
-  if (msm_tails(buckets, sh, halves ? 1 : nmsm, out_affine, out_xyzz, prof, st)) return 1;
-  if (prof) cudaEventRecord(g.ev[6], st);
-  BP_CUDA(cudaGetLastError());
-  return 0;
-}
-
-// ---- single large MSM, windows pipelined over streams -----------------------------------------------
-// After the sort, windows are accumulated top-down on two alternating streams; each window's bucket reduction runs
-// on its own (high-priority) stream as soon as that window's buckets are final, and one more stream folds the window
-// sums into the Horner accumulator.  The latency-bound tail kernels (a few hundred dependent point operations on a
-// handful of SMs) thereby run underneath the accumulation of the lower windows; only the last window's reduction, one
-// Horner step and the final inversion remain exposed.  Same kernels, same result as msm_run.
-static int msm_run_pipelined(const Affine* points, const u32* point_idx, const Fq* scalars, u32 T, Affine* out_affine, XYZZ* out_xyzz) {
-  cudaStream_t st = g.stream;
-  MsmShape sh = msm_shape(T, 1, g.force_c);
-  g.last_c = sh.c;
-  const size_t W = sh.U, nb = W * sh.H;      // W counts bucket units here (the top window may own two)
-  g.last_nb = nb;
-  if (T >= (1u << 30)) return fail("msm: too many terms");
-  if (g.ensure_pipeline((int)W)) return 1;
-  if (!g.pipe_attr_set && g.pipe_acc_smem) {   // optional cap of resident accumulate blocks per SM
-    BP_CUDA(cudaFuncSetAttribute(k_accumulate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.pipe_acc_smem));
-    g.pipe_attr_set = true;
-  }
-  int* digits = (int*)g.ws_digits.ensure((size_t)sh.W * 2 * T * sizeof(int));
-  uint2* entries = (uint2*)g.ws_entries.ensure((size_t)sh.W * 2 * T * sizeof(uint2));
-  Affine* phi = (Affine*)g.ws_phi.ensure((size_t)T * sizeof(Affine));
-  u32* count = (u32*)g.ws_count.ensure((nb + 1) * sizeof(u32));
-  u32* start = (u32*)g.ws_start.ensure((nb + 1) * sizeof(u32));
-  u32* cursor = (u32*)g.ws_cursor.ensure((nb + 1) * sizeof(u32));
-  size_t ntiles = (nb + 1 + BP_SCAN_TILE - 1) / BP_SCAN_TILE;
-  u32* tiles = (u32*)g.ws_tiles.ensure(ntiles * sizeof(u32));
-  XYZZ* buckets = (XYZZ*)g.ws_buckets.ensure(nb * sizeof(XYZZ));
-  XYZZ* segsum = (XYZZ*)g.ws_segsum.ensure(W * sh.nseg * sizeof(XYZZ));
-  XYZZ* seg_run = (XYZZ*)g.ws_segrun.ensure(W * sh.nseg * sizeof(XYZZ));
-  u32 G = sh.nseg < 8 ? sh.nseg : 8, ngrp = sh.nseg / G;
-  XYZZ* grpsum = (XYZZ*)g.ws_grpsum.ensure(W * ngrp * sizeof(XYZZ));
-  XYZZ* winsum = (XYZZ*)g.ws_winsum.ensure((W + 1) * sizeof(XYZZ));
-  XYZZ* hacc = winsum + W;                                   // Horner accumulator
-  const size_t wchunks = ((size_t)2 * T + sh.chunk - 1) / sh.chunk + 1;      // a window holds at most 2T entries
-  XYZZ* part = (XYZZ*)g.ws_part.ensure(2 * W * wchunks * sizeof(XYZZ));
-  const u32 big_cap = (u32)((size_t)2 * T / ((size_t)sh.chunk * (BP_FIXUP_SERIAL_MAX - 1)) + 16);
-  u32* big = (u32*)g.ws_big.ensure(W * (2 * (size_t)big_cap + 2) * sizeof(u32));
-  if (!digits || !entries || !phi || !count || !start || !cursor || !tiles || !buckets || !segsum || !seg_run || !grpsum || !winsum || !part || !big)
-    return fail("workspace allocation failed");
-  int lgS = 0, lgG = 0, ubits = 0;
-  while ((1u << lgS) < sh.S) lgS++;
-  while ((1u << lgG) < G) lgG++;
-  while ((1u << ubits) < ngrp * (1u + sh.dbl)) ubits++;
-
-  if (g.profiling) cudaEventRecord(g.ev[0], st);
-  BP_CUDA(cudaMemsetAsync(count, 0, (nb + 1) * sizeof(u32), st));
-  BP_CUDA(cudaMemsetAsync(big, 0, W * (2 * (size_t)big_cap + 2) * sizeof(u32), st));
+  if (opt.pts_ready) BP_CUDA(cudaStreamWaitEvent(st, opt.pts_ready, 0));   // points may still be uploading
   ++g.nlaunch, k_phi<<<(T + 127) / 128, 128, 0, st>>>(points, point_idx, T, phi);
-  ++g.nlaunch, k_digits<<<(T + 255) / 256, 256, 0, st>>>(scalars, T, nullptr, 1, sh, digits, count, nullptr, 0);
-  ++g.nlaunch, k_scan_tiles<<<(unsigned)ntiles, 256, 0, st>>>(count, start, tiles, nb + 1);
-  ++g.nlaunch, k_scan_sums<<<1, 1024, 0, st>>>(tiles, ntiles);
-  ++g.nlaunch, k_scan_add<<<(unsigned)ntiles, 256, 0, st>>>(start, tiles, nb + 1, nullptr);
-  BP_CUDA(cudaMemcpyAsync(cursor, start, (nb + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
-  ++g.nlaunch, k_scatter<<<(2 * T + 255) / 256, 256, 0, st>>>(digits, T, nullptr, 1, sh, cursor, entries);
-  BP_CUDA(cudaMemsetAsync(buckets, 0, nb * sizeof(XYZZ), st));
-  BP_CUDA(cudaEventRecord(g.pe_prep, st));
-  BP_CUDA(cudaStreamWaitEvent(g.ps_acc[0], g.pe_prep, 0));
-  BP_CUDA(cudaStreamWaitEvent(g.ps_acc[1], g.pe_prep, 0));
-  int k = 0;
-  for (int w = (int)W - 1; w >= 0; w--, k++) {
-    cudaStream_t sa = g.ps_acc[k & 1], sr = g.ps_red[w], shh = g.ps_hor;
-    const u32* gs = start + (size_t)w * sh.H;
-    XYZZ* part_w = part + 2 * (size_t)w * wchunks;
-    u32* big_w = big + (size_t)w * (2 * (size_t)big_cap + 2);
-    ++g.nlaunch, k_accumulate<<<(unsigned)((wchunks + 127) / 128), 128, g.pipe_acc_smem, sa>>>(points, point_idx, phi, start, entries, gs, gs + sh.H, sh.chunk, buckets, part_w);
-    BP_CUDA(cudaEventRecord(g.pe_acc[w], sa));
-    BP_CUDA(cudaStreamWaitEvent(sr, g.pe_acc[w], 0));
-    // everything after the accumulation of window w is a latency chain on few SMs: it lives on the window's own stream
-    ++g.nlaunch, k_fixup<<<(unsigned)((sh.H + 63) / 64), 64, 0, sr>>>(start, (size_t)w * sh.H, sh.H, gs, sh.chunk, part_w, buckets, big_w, big_cap);
-    ++g.nlaunch, k_fixup_mid<<<16, 256, 0, sr>>>(start, gs, sh.chunk, part_w, buckets, big_w, big_cap);
-    ++g.nlaunch, k_fixup_big<<<32, 64, 0, sr>>>(start, gs, sh.chunk, part_w, buckets, big_w);
-    const XYZZ* bw = buckets + (size_t)w * sh.H;
-    ++g.nlaunch, k_reduce_seg<<<(unsigned)((4 * (size_t)sh.nseg + 31) / 32), 32, 0, sr>>>(bw, sh, 1, seg_run + (size_t)w * sh.nseg, segsum + (size_t)w * sh.nseg);
-    ++g.nlaunch, k_reduce_grp<<<(unsigned)((4 * (size_t)ngrp + 31) / 32), 32, 0, sr>>>(seg_run + (size_t)w * sh.nseg, segsum + (size_t)w * sh.nseg, sh, 1, (u32)w, G, lgS, lgG,
-                                                                              ubits, grpsum + (size_t)w * ngrp);
-    if (ngrp > 1) ++g.nlaunch, k_window_sum<<<1, 64, 0, sr>>>(grpsum + (size_t)w * ngrp, ngrp, winsum + w);
-    else BP_CUDA(cudaMemcpyAsync(winsum + w, grpsum + (size_t)w * ngrp, sizeof(XYZZ), cudaMemcpyDeviceToDevice, sr));
-    BP_CUDA(cudaEventRecord(g.pe_red[w], sr));
-    BP_CUDA(cudaStreamWaitEvent(shh, g.pe_red[w], 0));
-    ++g.nlaunch, k_horner_step<<<1, 32, 0, shh>>>(hacc, winsum + w, (sh.dbl && w == (int)W - 2) ? 0 : sh.c, w == (int)W - 1 ? 1 : 0);
-  }
-  ++g.nlaunch, k_finish<<<1, 32, 0, g.ps_hor>>>(hacc, out_affine, out_xyzz);
-  BP_CUDA(cudaEventRecord(g.pe_done, g.ps_hor));
-  BP_CUDA(cudaStreamWaitEvent(st, g.pe_done, 0));
-  // the accumulate streams also rejoin (their last events precede pe_done through the dependency chain)
-  if (g.profiling) { for (int i = 1; i <= 6; i++) cudaEventRecord(g.ev[i], st); }
+  // E (= start[nb]) stays on the device: launch for the upper bound W*T, threads past E exit at once
+  if (prof) cudaEventRecord(g.ev_k0, st);
+  if (use_slots) ++g.nlaunch, k_accumulate_slots<true><<<(unsigned)((nchunks + 127) / 128), 128, 0, st>>>(points, phi, start, (u32)nb, slots, cap, overflow, sh.chunk, buckets, part);
+  ++g.nlaunch, k_accumulate<<<(unsigned)((nchunks + 127) / 128), 128, 0, st>>>(points, point_idx, phi, start, entries, zero_word, start + nb, sh.chunk, buckets, part, 0, 0, overflow);
+  if (prof) cudaEventRecord(g.ev_k1, st);
+  ++g.nlaunch, k_fixup<<<(unsigned)((nb + 127) / 128), 128, 0, st>>>(start, 0, nb, zero_word, sh.chunk, part, buckets, big, big_cap);
+  ++g.nlaunch, k_fixup_mid<<<2 * g.sm_count, 256, 0, st>>>(start, zero_word, sh.chunk, part, buckets, big, big_cap);
+  ++g.nlaunch, k_fixup_big<<<g.sm_count, 256, 0, st>>>(start, zero_word, sh.chunk, part, buckets, big);
+  if (prof) cudaEventRecord(g.ev[4], st);
+  if (msm_tails(buckets, sh, nmsm, out_affine, out_xyzz, prof, st)) return 1;
+  if (prof) cudaEventRecord(g.ev[6], st);
   BP_CUDA(cudaGetLastError());
   return 0;
 }
@@ -431,7 +278,6 @@ static int msm_run_pre(const Affine* pre, u32 stride, u32 first, int c, const Fq
   sh.c = c; sh.W = 1; sh.U = 1; sh.dbl = 0; sh.H = ps.H;
   const double ent_bound = (double)ps.W * (double)T;
   sh.chunk = acc_chunk(ent_bound);
-  if (g.pre_chunk) sh.chunk = g.pre_chunk;
   sh.seg_plain = (double)sh.H / 4 >= 32768.0 ? 1 : 0;
   sh.S = sh.seg_plain ? 4 : (sh.H < 8 ? sh.H : 8);
   sh.nseg = sh.H / sh.S;
@@ -445,33 +291,9 @@ static int msm_run_pre(const Affine* pre, u32 stride, u32 first, int c, const Fq
   }
   if ((unsigned long long)ps.W * stride >= (1ull << 30)) return fail("msm: too many terms for 30-bit point indices");
   const size_t nb = sh.H, emax = (size_t)ps.W * T;
-  // batched-affine pair passes ahead of the XYZZ accumulation (affine.cuh): OFF unless bp_msm_set_affine_passes asks for them.
-  // Measured at 2^20 (profiles/r2_affine_passes.txt): passes 1.44 + 0.64 + 0.35 ms + 0.24 ms XYZZ remainder against 1.80 ms for
-  // the XYZZ accumulation alone -- a shared inversion costs ~18-40 k warp instructions whoever executes it, and one MSM of this
-  // size has only ~250 k warp-level additions per pass to spread it over (DESIGN.md 5).
-  int P = g.aff_passes > 0 ? g.aff_passes : 0;
-  if (P > 6) P = 6;
-  const u32 amask = (1u << P) - 1u;
-  const size_t emax_pad = P ? emax + nb * amask : emax;                 // every bucket rounded up to a multiple of 2^P entries
-  if (emax_pad >= 0xFFFFFFF0ull) return fail("msm: too many entries");
-  if (P) {                                                              // the XYZZ stage sees 1/2^P of the entries
-    const double red = (double)(emax_pad >> P);
-    sh.chunk = acc_chunk(red);
-    if (g.pre_chunk) sh.chunk = g.pre_chunk;
-  }
-  const size_t nchunks = ((P ? (emax_pad >> P) : emax) + sh.chunk - 1) / sh.chunk;
-  int* digits = g.pre_fused ? nullptr : (int*)g.ws_digits.ensure(emax * sizeof(int));      // fused: the scatter pass recomputes the digits
-  uint2* entries = (uint2*)g.ws_entries.ensure(emax_pad * sizeof(uint2));
-  Affine *aff_a = nullptr, *aff_b = nullptr; Fp* aff_scr = nullptr; u32 *aff_ctr = nullptr, *red_start = nullptr; uint2* red_ent = nullptr;
-  if (P) {
-    aff_a = (Affine*)g.ws_aff_a.ensure((emax_pad / 2 + 1) * sizeof(Affine));
-    aff_b = (Affine*)g.ws_aff_b.ensure((emax_pad / 4 + 1) * sizeof(Affine));
-    aff_scr = (Fp*)g.ws_aff_scr.ensure((size_t)4 * g.sm_count * 128 * BP_AFF_B * sizeof(Fp));
-    aff_ctr = (u32*)g.ws_aff_ctr.ensure(8 * sizeof(u32));
-    red_start = (u32*)g.ws_aff_start.ensure((nb + 1) * sizeof(u32));
-    red_ent = (uint2*)g.ws_aff_ent.ensure(((emax_pad >> P) + 1) * sizeof(uint2));
-    if (!aff_a || !aff_b || !aff_scr || !aff_ctr || !red_start || !red_ent) return fail("workspace allocation failed");
-  }
+  if (emax >= 0xFFFFFFF0ull) return fail("msm: too many entries");
+  const size_t nchunks = (emax + sh.chunk - 1) / sh.chunk;
+  uint2* entries = (uint2*)g.ws_entries.ensure(emax * sizeof(uint2));
   u32* count = (u32*)g.ws_count.ensure((nb + 1) * sizeof(u32));
   u32* start = (u32*)g.ws_start.ensure((nb + 1) * sizeof(u32));
   u32* cursor = (u32*)g.ws_cursor.ensure((nb + 1) * sizeof(u32));
@@ -481,11 +303,11 @@ static int msm_run_pre(const Affine* pre, u32 stride, u32 first, int c, const Fq
   XYZZ* part = (XYZZ*)g.ws_part.ensure(2 * nchunks * sizeof(XYZZ));
   const u32 big_cap = (u32)(emax / ((size_t)sh.chunk * (BP_FIXUP_SERIAL_MAX - 1)) + 16);
   u32* big = (u32*)g.ws_big.ensure((2 * (size_t)big_cap + 4) * sizeof(u32));
-  if ((!digits && !g.pre_fused) || !entries || !count || !start || !cursor || !tiles || !buckets || !part || !big) return fail("workspace allocation failed");
+  if (!entries || !count || !start || !cursor || !tiles || !buckets || !part || !big) return fail("workspace allocation failed");
   u32* zero_word = big + 2 * (size_t)big_cap + 3;
   // slot sort (msm.cuh): one scattered pass instead of histogram + scatter for large MSMs; the exact counting sort stays queued
   // behind it as the fallback, gated on the overflow word
-  const bool use_slots = g.pre_slots > 0 && P == 0 && T >= g.pre_slots_min;
+  const bool use_slots = g.pre_slots > 0 && T >= g.pre_slots_min;
   u32 cap = 0; u32* slots = nullptr; u32* overflow = nullptr;
   if (use_slots) {
     double lam = 0;                                                      // mean load of the fullest buckets: the low ones, which every window reaches
@@ -500,41 +322,25 @@ static int msm_run_pre(const Affine* pre, u32 stride, u32 first, int c, const Fq
   BP_CUDA(cudaMemsetAsync(count, 0, (nb + 1) * sizeof(u32), st));
   if (prof) cudaEventRecord(g.ev[0], st);
   if (use_slots) ++g.nlaunch, k_scatter_slots_pre<4><<<(T + 255) / 256, 256, 0, st>>>(scalars, T, ps, stride, first, cap, count, slots, overflow);
-  else ++g.nlaunch, k_digits_pre<<<(T + 255) / 256, 256, 0, st>>>(scalars, T, ps, digits, count);
+  else ++g.nlaunch, k_digits_pre<<<(T + 255) / 256, 256, 0, st>>>(scalars, T, ps, count);
   if (prof) cudaEventRecord(g.ev[1], st);
-  ++g.nlaunch, k_scan_tiles<<<(unsigned)ntiles, 256, 0, st>>>(count, start, tiles, nb + 1, amask);
+  ++g.nlaunch, k_scan_tiles<<<(unsigned)ntiles, 256, 0, st>>>(count, start, tiles, nb + 1);
   ++g.nlaunch, k_scan_sums<<<1, 1024, 0, st>>>(tiles, ntiles);
   ++g.nlaunch, k_scan_add<<<(unsigned)ntiles, 256, 0, st>>>(start, tiles, nb + 1, nullptr);
   if (prof) cudaEventRecord(g.ev[2], st);
   BP_CUDA(cudaMemcpyAsync(cursor, start, (nb + 1) * sizeof(u32), cudaMemcpyDeviceToDevice, st));
-  if (P) ++g.nlaunch, k_aff_pad<<<(unsigned)((nb + 255) / 256), 256, 0, st>>>(start, count, (u32)nb, entries);
-  ++g.nlaunch, k_scatter_pre<<<(T + 255) / 256, 256, 0, st>>>(use_slots ? nullptr : digits, scalars, T, ps, stride, first, cursor, entries, overflow);
+  ++g.nlaunch, k_scatter_pre<<<(T + 255) / 256, 256, 0, st>>>(scalars, T, ps, stride, first, cursor, entries, overflow);
   if (prof) cudaEventRecord(g.ev[3], st);
   BP_CUDA(cudaMemsetAsync(buckets, 0, nb * sizeof(XYZZ), st));
   BP_CUDA(cudaMemsetAsync(zero_word, 0, sizeof(u32), st));
   BP_CUDA(cudaMemsetAsync(big, 0, 2 * sizeof(u32), st));
   if (prof) cudaEventRecord(g.ev_k0, st);
-  const Affine* acc_pts = pre; const u32* acc_start = start; const uint2* acc_ent = entries;
-  if (P) {
-    // batched-affine pair passes (affine.cuh): the list halves P times, then the XYZZ accumulation takes over at 1/2^P of the additions
-    BP_CUDA(cudaMemsetAsync(aff_ctr, 0, 8 * sizeof(u32), st));
-    const unsigned grid = 4 * (unsigned)g.sm_count;
-    const Affine* src = nullptr;
-    for (int p = 0; p < P; p++) {
-      Affine* dst = (p & 1) ? aff_b : aff_a;
-      if (p == 0) ++g.nlaunch, k_aff_pass<BP_AFF_B, true><<<grid, 128, 0, st>>>(pre, nullptr, nullptr, entries, nullptr, start + nb, 0, dst, aff_scr, aff_ctr);
-      else ++g.nlaunch, k_aff_pass<BP_AFF_B, false><<<grid, 128, 0, st>>>(nullptr, nullptr, nullptr, nullptr, src, start + nb, (u32)p, dst, aff_scr, aff_ctr + p);
-      src = dst;
-    }
-    ++g.nlaunch, k_aff_index<<<(unsigned)(((emax_pad >> P) > nb + 1 ? (emax_pad >> P) : nb + 1) + 255) / 256, 256, 0, st>>>(start, (u32)nb, entries, P, red_start, red_ent);
-    acc_pts = src; acc_start = red_start; acc_ent = red_ent;
-  }
   if (use_slots) ++g.nlaunch, k_accumulate_slots<false><<<(unsigned)((nchunks + 127) / 128), 128, 0, st>>>(pre, nullptr, start, (u32)nb, slots, cap, overflow, sh.chunk, buckets, part);
-  ++g.nlaunch, k_accumulate<<<(unsigned)((nchunks + 127) / 128), 128, 0, st>>>(acc_pts, nullptr, nullptr, acc_start, acc_ent, zero_word, acc_start + nb, sh.chunk, buckets, part, 0, 0, overflow);
+  ++g.nlaunch, k_accumulate<<<(unsigned)((nchunks + 127) / 128), 128, 0, st>>>(pre, nullptr, nullptr, start, entries, zero_word, start + nb, sh.chunk, buckets, part, 0, 0, overflow);
   if (prof) cudaEventRecord(g.ev_k1, st);
-  ++g.nlaunch, k_fixup<<<(unsigned)((nb + 127) / 128), 128, 0, st>>>(acc_start, 0, nb, zero_word, sh.chunk, part, buckets, big, big_cap);
-  ++g.nlaunch, k_fixup_mid<<<2 * g.sm_count, 256, 0, st>>>(acc_start, zero_word, sh.chunk, part, buckets, big, big_cap);
-  ++g.nlaunch, k_fixup_big<<<g.sm_count, 256, 0, st>>>(acc_start, zero_word, sh.chunk, part, buckets, big);
+  ++g.nlaunch, k_fixup<<<(unsigned)((nb + 127) / 128), 128, 0, st>>>(start, 0, nb, zero_word, sh.chunk, part, buckets, big, big_cap);
+  ++g.nlaunch, k_fixup_mid<<<2 * g.sm_count, 256, 0, st>>>(start, zero_word, sh.chunk, part, buckets, big, big_cap);
+  ++g.nlaunch, k_fixup_big<<<g.sm_count, 256, 0, st>>>(start, zero_word, sh.chunk, part, buckets, big);
   if (prof) cudaEventRecord(g.ev[4], st);
   if (sh.H < 4096) {                                   // small unit: the running-sum tails of the plain path
     if (msm_tails(buckets, sh, 1, out_affine, out_xyzz, prof, st)) return 1;
@@ -546,8 +352,7 @@ static int msm_run_pre(const Affine* pre, u32 stride, u32 first, int c, const Fq
     // K = 8 for the 2^17-bucket unit of large MSMs, 4 below (gpurun_out/prek.log: 2^16 terms, c = 17: K = 8 / 4 / 2 -> 0.432 / 0.416 /
     // 0.414 ms, the first level is a latency chain of K - 1 lone-thread additions there; 2^20 terms, c = 18: 2.268 / 2.284 / 2.303 ms,
     // twice the partial sums cost the weighted stage more than the shorter first level saves)
-    static const u32 Kenv = [] { const char* e = getenv("BP_PRE_K"); int v = e ? atoi(e) : 0; return (u32)(v == 8 || v == 4 || v == 2 ? v : 0); }();
-    const u32 Kpre = Kenv ? Kenv : (sh.H >= (1u << 17) ? 8u : 4u);
+    const u32 Kpre = sh.H >= (1u << 17) ? 8u : 4u;
     const u32 Kr = C >= Kpre ? Kpre : C, Kc = R >= Kpre ? Kpre : R;
     const u32 np_r = C / Kr, np_c = R / Kc;              // partial sums per row / per column
     XYZZ* ping = (XYZZ*)g.ws_segsum.ensure(((size_t)nb / Kr + (size_t)nb / Kc + 8192) * sizeof(XYZZ));
@@ -571,7 +376,7 @@ static int msm_run_pre(const Affine* pre, u32 stride, u32 first, int c, const Fq
 
 // Host operands -> device: scalars first on the compute stream (the digit/sort stages only need them), points on a
 // second stream so that their (twice as large) upload overlaps those stages; msm_run waits for the points right
-// before the first kernel that reads them.  The pipelined/profiling paths simply wait up front.
+// before the first kernel that reads them.
 // Large host -> device copies go down in pieces: on the B200 hosts measured here one cudaMemcpyAsync of 32-96 MiB from pinned
 // memory runs at 18-38 GB/s, the same bytes as <= 8 MiB copies back to back at 52 GB/s (tools/h2d_probe.py, profiles/r2_h2d_probe.txt).
 static size_t h2d_piece() {
@@ -591,34 +396,24 @@ static int upload_operands(Affine* d_pts, const uint8_t* pts64, Fq* d_sc, const 
   *opt = MsmOpts();
   BP_CUDA(cudaEventRecord(g.ev_copy_gate, g.stream));                     // earlier work may still read d_pts
   BP_CUDA(cudaStreamWaitEvent(g.copy_stream, g.ev_copy_gate, 0));
-  if (n >= ((size_t)1 << 17) && g.force_c == 0 && !g.profiling && n < g.pipeline_min_terms) {
-    // big MSM: everything on the copy stream in the order it is needed -- scalars, then the points in K equal parts -- msm_run
-    // sorts as soon as the scalars are in and accumulates part by part into one set of buckets (see there).  K = 4: the
-    // accumulation of a quarter (0.49 ms) roughly matches its upload (0.44 ms at the 36-38 GB/s this host sustains), so the GPU
-    // neither waits for the last part nor starts late (profiles/r2_e2e_timeline.txt)
+  if (n >= ((size_t)1 << 17) && g.force_c == 0 && !g.profiling) {
+    // big MSM: everything on the copy stream in the order it is needed -- per part its scalars, then its points -- and
+    // msm_run_parts sorts each part as soon as its scalars are in and accumulates it into one set of buckets as soon as its
+    // points are.  K = 4: the accumulation of a quarter (0.49 ms) roughly matches its upload (0.44 ms at the 36-38 GB/s this host
+    // sustains), so the GPU neither waits for the last part nor starts late (profiles/r2_e2e_timeline.txt)
     static const int parts = [] { const char* e = getenv("BP_E2E_PARTS"); int v = e ? atoi(e) : 4; return v >= 2 && v <= 8 ? v : 4; }();
-    static const bool split_sort = [] { const char* e = getenv("BP_E2E_ONE_SORT"); return !(e && atoi(e)); }();
-    opt->parts = parts; opt->split_sort = split_sort;
+    opt->parts = parts;
     g.dbg_rec(0, g.copy_stream);
-    if (!split_sort) {
-      BP_CUDA(h2d_chunked(d_sc, sc32, n * 32, g.copy_stream));
-      g.dbg_rec(1, g.copy_stream);
-    }
-    BP_CUDA(cudaEventRecord(g.ev_sc, g.copy_stream));
-    for (int k = 0; k < parts; k++) {                      // part k = terms [n*k/K, n*(k+1)/K)  (the same cut as msm_run's)
+    for (int k = 0; k < parts; k++) {                      // part k = terms [n*k/K, n*(k+1)/K)  (the same cut as msm_run_parts')
       const size_t lo = (size_t)((unsigned long long)n * k / parts), hi = (size_t)((unsigned long long)n * (k + 1) / parts);
-      if (split_sort) {                                    // the part's scalars first: its sort starts while its points are on the wire
-        BP_CUDA(h2d_chunked(d_sc + lo, sc32 + lo * 32, (hi - lo) * 32, g.copy_stream));
-        BP_CUDA(cudaEventRecord(g.ev_part_sc[k], g.copy_stream));
-        if (k == 0) g.dbg_rec(1, g.copy_stream);
-      }
+      BP_CUDA(h2d_chunked(d_sc + lo, sc32 + lo * 32, (hi - lo) * 32, g.copy_stream));
+      BP_CUDA(cudaEventRecord(g.ev_part_sc[k], g.copy_stream));
+      if (k == 0) g.dbg_rec(1, g.copy_stream);
       BP_CUDA(h2d_chunked(d_pts + lo, pts64 + lo * 64, (hi - lo) * 64, g.copy_stream));
       BP_CUDA(cudaEventRecord(g.ev_half[k], g.copy_stream));
       if (k == 0) g.dbg_rec(2, g.copy_stream);
       if (k == parts - 1) g.dbg_rec(3, g.copy_stream);
     }
-    BP_CUDA(cudaStreamWaitEvent(g.stream, g.ev_sc, 0));
-    opt->halves = true;
     return 0;
   }
   BP_CUDA(h2d_chunked(d_sc, sc32, n * 32, g.stream));
@@ -821,14 +616,12 @@ int bp_init(int device) {
   BP_CUDA(cudaGetDeviceProperties(&prop, device));
   if (prop.major < 10) return fail("bp_init: device %s is sm_%d%d; this library is built for sm_100a only", prop.name, prop.major, prop.minor);
   g.device = device; g.sm_count = prop.multiProcessorCount;
-  acc_slots() = (unsigned)g.sm_count * BP_ACC_MINB * 128u;
   BP_CUDA(cudaStreamCreateWithFlags(&g.stream, cudaStreamNonBlocking));
   for (int i = 0; i < 8; i++) BP_CUDA(cudaEventCreate(&g.ev[i]));
   BP_CUDA(cudaEventCreate(&g.ev_a)); BP_CUDA(cudaEventCreate(&g.ev_b));
   BP_CUDA(cudaEventCreate(&g.ev_k0)); BP_CUDA(cudaEventCreate(&g.ev_k1));
   BP_CUDA(cudaStreamCreateWithFlags(&g.copy_stream, cudaStreamNonBlocking));
   BP_CUDA(cudaEventCreateWithFlags(&g.ev_pts, cudaEventDisableTiming)); BP_CUDA(cudaEventCreateWithFlags(&g.ev_copy_gate, cudaEventDisableTiming));
-  BP_CUDA(cudaEventCreateWithFlags(&g.ev_sc, cudaEventDisableTiming));
   for (int i = 0; i < 8; i++) BP_CUDA(cudaEventCreateWithFlags(&g.ev_half[i], cudaEventDisableTiming));
   for (int i = 0; i < 8; i++) BP_CUDA(cudaEventCreateWithFlags(&g.ev_part_sc[i], cudaEventDisableTiming));
   g.inited = true;
@@ -882,9 +675,6 @@ int bp_msm_last_entries(uint64_t* entries) {      // non-zero digits = mixed add
   return 0;
 }
 int bp_launch_count(uint64_t* launches) { *launches = g.nlaunch; return 0; }
-int bp_msm_set_affine_passes(int passes) { g.aff_passes = passes < 0 ? -1 : (passes > 6 ? 6 : passes); return 0; }   /* experiment switch */
-int bp_msm_set_tails2d(int on) { g.tails2d = on != 0; return 0; }   /* experiment switch */
-int bp_msm_set_pre_fused(int on) { if (g.inited) cudaStreamSynchronize(g.stream); g.pre_fused = on != 0; pre_graphs_clear(); return 0; }   /* experiment switch */
 int bp_msm_set_pre_slots(int mode, size_t min_terms) {   /* 0 = exact counting sort only, 1 = slot sort for MSMs of >= min_terms terms (0 = keep), 2 = same with 8 slots per bucket (test hook: forces the fallback) */
   if (g.inited) cudaStreamSynchronize(g.stream);
   g.pre_slots = mode; if (min_terms) g.pre_slots_min = (unsigned)min_terms;
@@ -893,9 +683,7 @@ int bp_msm_set_pre_slots(int mode, size_t min_terms) {   /* 0 = exact counting s
   return 0;
 }
 int bp_msm_set_host_finish(int on) { g.hf_enabled = on != 0; return 0; }   /* 1 (default): host-result MSMs of the plain path finish their Horner chain on the host */
-int bp_msm_set_pre_chunk(int entries) { g.pre_chunk = entries > 0 ? (unsigned)entries : 0; return 0; }   /* experiment switch */
 int bp_msm_set_profiling(int on) { g.profiling = on != 0; return 0; }
-int bp_msm_set_pipeline_min(size_t min_terms) { g.pipeline_min_terms = min_terms ? (unsigned)min_terms : 0xFFFFFFFFu; return 0; }
 int bp_msm_stage_ms(float out7[7]) {
   BP_NEED_INIT();
   BP_CUDA(cudaStreamSynchronize(g.stream));
@@ -982,7 +770,7 @@ static unsigned long long g_pre_graph_clock = 0;
 static bool g_small_graphs = true;
 static void pre_graphs_clear() { for (auto& e : g_pre_graphs) if (e.exec) cudaGraphExecDestroy(e.exec); g_pre_graphs.clear(); }
 static int msm_run_pre_small(const Affine* pre, u32 stride, u32 first, int c, const Fq* scalars, u32 T, Affine* out_affine, XYZZ* out_xyzz) {
-  if (!g_small_graphs || T == 0 || T > (1u << 17) || g.profiling || g.aff_passes > 0 || g.pre_chunk)
+  if (!g_small_graphs || T == 0 || T > (1u << 17) || g.profiling)
     return msm_run_pre(pre, stride, first, c, scalars, T, out_affine, out_xyzz);
   PreGraph* hit = nullptr;
   for (auto& e : g_pre_graphs)
@@ -1035,12 +823,6 @@ static int handle_msm(const HandleRec& P, size_t first, const Fq* d_sc, size_t n
   return msm_run((const Affine*)P.p + first, nullptr, d_sc, (u32)n, nullptr, 1, n, out_affine, out_xyzz);
 }
 
-extern "C" int bp_msm_set_chunk_fit(int on) {   /* experiment switch; cached small-MSM graphs carry the chunk they were captured with */
-  acc_chunk_fit() = on ? 1 : 0;
-  if (g.inited) cudaStreamSynchronize(g.stream);
-  pre_graphs_clear();
-  return 0;
-}
 extern "C" int bp_msm_set_small_graphs(int on) { g_small_graphs = on != 0; if (!on) { if (g.inited) cudaStreamSynchronize(g.stream); pre_graphs_clear(); } return 0; }
 
 static int handle_msm_to_host(const HandleRec& P, size_t first, const Fq* d_sc, size_t n, uint8_t* out64) {

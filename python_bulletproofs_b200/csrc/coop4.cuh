@@ -31,6 +31,12 @@ BP_DI Fp shfl_down_fp(const Fp& m, int delta) {
   for (int i = 0; i < 8; i++) r.v[i] = __shfl_down_sync(BP_FULL_MASK, m.v[i], delta);
   return r;
 }
+BP_DI Fp shfl_up_fp(const Fp& m, int delta) {
+  Fp r;
+#pragma unroll
+  for (int i = 0; i < 8; i++) r.v[i] = __shfl_up_sync(BP_FULL_MASK, m.v[i], delta);
+  return r;
+}
 BP_DI Fp sel_fp(bool c, const Fp& a, const Fp& b) {
   Fp r;
 #pragma unroll

@@ -45,25 +45,19 @@ struct Ctx {
   cudaEvent_t ev_a, ev_b, ev_k0, ev_k1;
   cudaStream_t copy_stream = nullptr;           // uploads of points overlap the scalar-only stages
   cudaEvent_t ev_pts = nullptr, ev_copy_gate = nullptr;
-  // large host-operand MSMs: the points arrive in two halves (ev_half[0], ev_half[1]); msm_run then runs the MSM as two
-  // half-size MSMs over one sort so that the first half is accumulated while the second is still on the wire
-  cudaEvent_t ev_half[8] = {nullptr}, ev_part_sc[8] = {nullptr}, ev_sc = nullptr;
-  DevBuf ws_halfoff;
+  // large host-operand MSMs: the operands arrive in K parts (upload_operands), part k's scalars at ev_part_sc[k] and its points
+  // at ev_half[k]; msm_run_parts sorts each part as its scalars land and accumulates it as its points land
+  cudaEvent_t ev_half[8] = {nullptr}, ev_part_sc[8] = {nullptr};
   cudaEvent_t dbg_ev[12] = {nullptr}; bool dbg_e2e = false;      // BP_E2E_TIMING: timeline of a host-operand MSM (development aid)
   void dbg_rec(int i, cudaStream_t st) { if (!dbg_e2e) return; if (!dbg_ev[i]) cudaEventCreate(&dbg_ev[i]); cudaEventRecord(dbg_ev[i], st); }
   bool profiling = false;
   int force_c = 0, last_c = 0;
-  bool pre_attr_set = false; unsigned pre_chunk = 0;
-  bool pre_fused = true;      // pre path: no digit array between the histogram and the scatter pass, the scatter recomputes the digits (bp_msm_set_pre_fused)
   // host-finished Horner (fp_host.h: horner_host): a host-result MSM on the plain path leaves its U window sums where `ws` points
   // instead of launching k_combine; the caller copies them out and finishes on a host core
   struct HostFinish { const void* ws = nullptr; int c = 0, W = 0, U = 0, dbl = 0; bool pending = false; } hf;
   bool hf_want = false, hf_enabled = true;
   int pre_slots = 1; unsigned pre_slots_min = 1u << 18; bool pre_slots_any = false;   // slot sort of the precomputed path (bp_msm_set_pre_slots)
   DevBuf ws_slots, ws_slots_ovf;
-  bool tails2d = false;       // 2-D marginal bucket reduction for the wide units of a large plain MSM (bp_msm_set_tails2d): measured slower, off
-  int aff_passes = -1;                          // batched-affine pair passes ahead of the XYZZ accumulation: <= 0 = off (default), 1..6 = that many passes (bp_msm_set_affine_passes)
-  DevBuf ws_aff_a, ws_aff_b, ws_aff_scr, ws_aff_ent, ws_aff_start, ws_aff_ctr;
   unsigned long long nlaunch = 0;               // kernels launched by this library so far (bp_launch_count)
   size_t last_nb = 0;
   // MSM workspaces
@@ -85,32 +79,6 @@ struct Ctx {
     }
     for (int i = 0; i < 2; i++)
       if (!var_done[i] && cudaEventCreateWithFlags(&var_done[i], cudaEventDisableTiming) != cudaSuccess) return fail("event creation failed");
-    return 0;
-  }
-  // pipelined single-MSM path: 2 accumulate streams, one reduce stream per window, one Horner stream
-  unsigned pipeline_min_terms = 0xFFFFFFFFu;   // off by default: on B200 the tail kernels starve behind the resident accumulate blocks (DESIGN.md 5)
-  cudaStream_t ps_acc[2] = {nullptr, nullptr}, ps_red[20] = {nullptr}, ps_hor = nullptr;
-  cudaEvent_t pe_prep = nullptr, pe_done = nullptr, pe_acc[20], pe_red[20];
-  int pipe_windows = 0;
-  size_t pipe_acc_smem = 0;             // >0 caps the accumulation at fewer resident blocks per SM (experiment: slower)
-  bool pipe_attr_set = false;
-  int ensure_pipeline(int W) {
-    if (W > 20) return fail("pipeline: too many windows");
-    if (!ps_hor) {
-      int lo = 0, hi = 0;
-      cudaDeviceGetStreamPriorityRange(&lo, &hi);
-      for (int i = 0; i < 2; i++) if (cudaStreamCreateWithPriority(&ps_acc[i], cudaStreamNonBlocking, lo) != cudaSuccess) return fail("stream creation failed");
-      if (cudaStreamCreateWithPriority(&ps_hor, cudaStreamNonBlocking, hi) != cudaSuccess) return fail("stream creation failed");
-      if (cudaEventCreateWithFlags(&pe_prep, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&pe_done, cudaEventDisableTiming) != cudaSuccess)
-        return fail("event creation failed");
-    }
-    for (; pipe_windows < W; pipe_windows++) {
-      int lo = 0, hi = 0;
-      cudaDeviceGetStreamPriorityRange(&lo, &hi);
-      if (cudaStreamCreateWithPriority(&ps_red[pipe_windows], cudaStreamNonBlocking, hi) != cudaSuccess) return fail("stream creation failed");
-      if (cudaEventCreateWithFlags(&pe_acc[pipe_windows], cudaEventDisableTiming) != cudaSuccess ||
-          cudaEventCreateWithFlags(&pe_red[pipe_windows], cudaEventDisableTiming) != cudaSuccess) return fail("event creation failed");
-    }
     return 0;
   }
   // pinned staging for the chunked batch verifier
@@ -219,8 +187,8 @@ struct Ctx {
   void free_all() {
     DevBuf* all[] = {&ws_pts, &ws_sc, &ws_off, &ws_out, &ws_digits, &ws_entries, &ws_count, &ws_start, &ws_cursor, &ws_tiles,
                      &ws_buckets, &ws_segsum, &ws_winsum, &ws_misc, &ws_flush, &ws_g, &ws_h, &ws_a, &ws_b, &ws_g2, &ws_h2,
-                     &ws_a2, &ws_b2, &ws_idx, &ws_lr, &ws_terms_sc, &ws_small, &ws_entry_bucket, &ws_part, &ws_big, &ws_phi, &ws_segrun, &ws_grpsum, &ws_winpart, &ws_fb_lanes, &ws_fb_var, &ws_sv_tab, &ws_sv_acc, &ws_sv_sc, &ws_rp_sums, &ws_halfoff,
-                     &ws_aff_a, &ws_aff_b, &ws_aff_scr, &ws_aff_ent, &ws_aff_start, &ws_aff_ctr, &ws_ipa_rp, &ws_ipa_ticket, &ws_slots, &ws_slots_ovf};
+                     &ws_a2, &ws_b2, &ws_idx, &ws_lr, &ws_terms_sc, &ws_small, &ws_entry_bucket, &ws_part, &ws_big, &ws_phi, &ws_segrun, &ws_grpsum, &ws_winpart, &ws_fb_lanes, &ws_fb_var, &ws_sv_tab, &ws_sv_acc, &ws_sv_sc, &ws_rp_sums,
+                     &ws_ipa_rp, &ws_ipa_ticket, &ws_slots, &ws_slots_ovf};
     rp_sums_src.clear();
     for (DevBuf* b : all) b->release();
   }

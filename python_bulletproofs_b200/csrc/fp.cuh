@@ -254,35 +254,14 @@ BP_DI void mul_wide_karatsuba(u32 t[16], const u32 a[8], const u32 b[8]) {
         "r"(mid[0]), "r"(mid[1]), "r"(mid[2]), "r"(mid[3]), "r"(mid[4]), "r"(mid[5]), "r"(mid[6]), "r"(mid[7]), "r"(mid[8]));
 }
 
-// BP_FOLD_DFMA = 1 moves the eight hi_i * 977 products of the fold to the FP64 pipe.  Measured on B200 and left OFF: fp_mul
-// 0.104 -> 0.100 T/s, fp_sqr 0.168 -> 0.124 T/s, k_accumulate 1.79 -> 2.08 ms at 2^20 -- the int <-> double register pairing and
-// the masks cost more issue slots than the 8 of 72 IMAD.WIDE they free (DESIGN.md 5, pipe measurements).
-#ifndef BP_FOLD_DFMA
-#define BP_FOLD_DFMA 0
-#endif
 // r = t mod p (lazy), t 512 bits:  t = lo + hi*2^256 = lo + hi*C
 BP_DI void fold512(u32 r[8], const u32 t[16]) {
   // hi * 977 as two sets of independent 32x32->64 products: se[2k..2k+1] = t[8+2k]*977 at limb 2k, so[2k..2k+1] =
   // t[9+2k]*977 at limb 2k+1.  Both sets live in aligned register pairs with no addend, so every product is a bare
   // IMAD.WIDE (a mad chain through the odd positions needed pairs that straddle two products: ~16 register moves per
   // fold on the multiplier pipe, the top non-arithmetic cost in the accumulation kernel's SASS).
+  // The same products on the FP64 pipe (DFMA on 2^52 + t) were measured slower: k_accumulate 1.79 -> 2.08 ms at 2^20 (DESIGN.md 5).
   u32 se[8], so[8];
-#if BP_FOLD_DFMA
-  // The eight products hi_i * 977 on the FP64 pipe, which issues side by side with the IMAD.WIDE pipe that bounds this code
-  // (profiles/r1_pipe_probe.txt, modes 10/11).  {0x43300000 : t} is the double 2^52 + t; fma(2^52 + t, 977, 2^52 - 977 * 2^52)
-  // = 2^52 + 977 t EXACTLY (one rounding of an integer below 2^53), whose mantissa holds the 42-bit product: low word = its low
-  // 32 bits, low 20 bits of the high word = its high bits.  One DFMA + one LOP3 per product instead of an IMAD.WIDE.
-  {
-    const double c977 = 977.0, coff = -976.0 * 4503599627370496.0;
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const double de = fma(__hiloint2double(0x43300000, (int)t[8 + 2 * k]), c977, coff);
-      const double dd = fma(__hiloint2double(0x43300000, (int)t[9 + 2 * k]), c977, coff);
-      se[2 * k] = (u32)__double2loint(de); se[2 * k + 1] = (u32)__double2hiint(de) & 0x000FFFFFu;
-      so[2 * k] = (u32)__double2loint(dd); so[2 * k + 1] = (u32)__double2hiint(dd) & 0x000FFFFFu;
-    }
-  }
-#else
   asm("mul.lo.u32 %0,%8,%12; mul.hi.u32 %1,%8,%12; mul.lo.u32 %2,%9,%12; mul.hi.u32 %3,%9,%12;"
       "mul.lo.u32 %4,%10,%12; mul.hi.u32 %5,%10,%12; mul.lo.u32 %6,%11,%12; mul.hi.u32 %7,%11,%12;"
       : "=r"(se[0]), "=r"(se[1]), "=r"(se[2]), "=r"(se[3]), "=r"(se[4]), "=r"(se[5]), "=r"(se[6]), "=r"(se[7])
@@ -291,7 +270,6 @@ BP_DI void fold512(u32 r[8], const u32 t[16]) {
       "mul.lo.u32 %4,%10,%12; mul.hi.u32 %5,%10,%12; mul.lo.u32 %6,%11,%12; mul.hi.u32 %7,%11,%12;"
       : "=r"(so[0]), "=r"(so[1]), "=r"(so[2]), "=r"(so[3]), "=r"(so[4]), "=r"(so[5]), "=r"(so[6]), "=r"(so[7])
       : "r"(t[9]), "r"(t[11]), "r"(t[13]), "r"(t[15]), "r"(977u));
-#endif
   // w = so + hi (both at limb 1), u = lo + se (limb 0): in these two chains ptxas folds each product into an
   // IMAD.WIDE whose 64-bit addend is an aligned pair; the third chain u += w << 32 is plain adds.
   u32 w[8], u[9], top, top2;

@@ -48,23 +48,9 @@ struct MsmShape {
 };
 #define BP_GLV_BITS 128
 
-// Entries per accumulation thread.  Every k_accumulate thread performs exactly `chunk` mixed additions and BP_ACC_MINB blocks
-// of 128 threads are resident per SM, so a launch runs in waves of acc_slots() threads that all end together: a last wave that
-// is only partly filled costs as much as a full one.  The chunk is therefore the smallest one that fills a whole number of
-// waves at the size class's target (8 / 16 / BP_CHUNK entries: small problems want short chains, large ones few partial sums).
-//   2^20 terms, c = 18 (pre path): 15.7 M entries / 32 = 6.49 waves -> 7 waves of 32 additions; at 30 entries the 7 waves are full.
-// Measured on B200 and left OFF (gpurun_out/chunkfit.log): 2^20 pre path 2.385 -> 2.407 ms (chunk 32 -> 30), e2e 2^20 3.476 -> 3.509 ms
-// (parts: 32 -> 28), 2^16 pre 0.422 -> 0.426 ms (8 -> 7) -- the blocks of a launch do not end together (gather latencies differ
-// from block to block), so the last wave is not a step, and the extra partial sums cost what the fit gains.
-inline unsigned& acc_slots() { static unsigned v = 148u * 512u; return v; }     // set from the device's SM count in bp_init
-inline int& acc_chunk_fit() { static int v = 0; return v; }                     // bp_msm_set_chunk_fit; OFF: measured no gain, see above
+// Entries per accumulation thread: small problems want short chains, large ones few partial sums.
 inline u32 acc_chunk(double entries) {
-  const u32 target = entries <= 1300000.0 ? 8 : (entries <= 2600000.0 ? 16 : BP_CHUNK);
-  const double slots = (double)acc_slots();
-  if (!acc_chunk_fit() || entries <= slots * target) return target;             // (less than one wave: nothing to fit)
-  const double waves = ceil(entries / (slots * target));
-  const u32 cl = (u32)ceil(entries / (waves * slots));
-  return cl < 4 ? 4 : cl;
+  return entries <= 1300000.0 ? 8 : (entries <= 2600000.0 ? 16 : BP_CHUNK);
 }
 
 inline MsmShape msm_shape(size_t terms_per_msm, size_t nmsm, int force_c = 0) {
@@ -242,13 +228,12 @@ __global__ void __launch_bounds__(128) k_phi(const Affine* __restrict__ points, 
 
 // ---- exclusive scan of u32 counts (3 passes; totals < 2^32) ---------------------------------------
 #define BP_SCAN_TILE 2048
-// amask = 2^P - 1 rounds every count up to a multiple of 2^P first (bucket starts aligned for the pair passes of affine.cuh)
-__global__ void __launch_bounds__(256) k_scan_tiles(const u32* __restrict__ in, u32* __restrict__ out, u32* __restrict__ tile_sum, size_t n, u32 amask = 0) {
+__global__ void __launch_bounds__(256) k_scan_tiles(const u32* __restrict__ in, u32* __restrict__ out, u32* __restrict__ tile_sum, size_t n) {
   __shared__ u32 sm[256];
   size_t base = (size_t)blockIdx.x * BP_SCAN_TILE + (size_t)threadIdx.x * 8;
   u32 v[8], s = 0;
 #pragma unroll
-  for (int i = 0; i < 8; i++) { v[i] = base + i < n ? (in[base + i] + amask) & ~amask : 0; s += v[i]; }
+  for (int i = 0; i < 8; i++) { v[i] = base + i < n ? in[base + i] : 0; s += v[i]; }
   sm[threadIdx.x] = s;
   __syncthreads();
   for (int off = 1; off < 256; off <<= 1) {
@@ -321,11 +306,11 @@ __global__ void __launch_bounds__(128, BP_ACC_MINB) k_accumulate(const Affine* _
                                                     XYZZ* __restrict__ buckets, XYZZ* __restrict__ part, u32 hb = 0, int into = 0,
                                                     const u32* __restrict__ run_if = nullptr) {
   if (run_if && __ldg(run_if) == 0) return;                              // fallback of the slot sort (k_scatter_slots_pre)
-  // hb / into: a host-operand MSM whose points arrive in K parts is sorted as K MSMs -- bucket id (part, unit, digit), hb
-  // buckets per part -- but all parts accumulate into ONE set of hb bucket values: the value of bucket id b lives at b % hb, and
-  // from the second part on (into = 1) the first piece of every bucket starts from the stored value instead of the identity.
-  // entry range [gs, ge) of this launch (all windows, or one window of the pipelined single-MSM path); both bounds
-  // are bucket_start[] words, read on the device so that no host round trip separates the sort from the accumulation
+  // hb / into: a host-operand MSM whose points arrive in K parts (msm_run_parts) sorts every part on its own over the same hb
+  // bucket ids, and all parts accumulate into ONE set of hb bucket values: from the second part on (into = 1) the first piece of
+  // every bucket starts from the stored value instead of the identity.
+  // entry range [gs, ge) of this launch: both bounds are bucket_start[] words, read on the device so that no host round trip
+  // separates the sort from the accumulation
   u32 chunk = blockIdx.x * blockDim.x + threadIdx.x;
   const u32 gs = __ldg(gs_ptr), E = __ldg(ge_ptr);
   u32 cs = gs + chunk * CL;
@@ -591,46 +576,20 @@ __global__ void __launch_bounds__(128) k_combine_plain(const XYZZ* __restrict__ 
   if (out) st_affine(out + m, xyzz_to_affine(acc));
 }
 
-// pipelined single-MSM path: acc <- 2^c * acc + winsum  (first: acc <- winsum), one quad
-__global__ void __launch_bounds__(32) k_horner_step(XYZZ* __restrict__ acc_io, const XYZZ* __restrict__ ws, int ndbl, int first) {
-  const int lane = threadIdx.x & 31, role = lane & 3, base = lane & ~3;
-  XYZZ v = ld_xyzz(ws);
-  XYZZ acc = v;
-  if (!first) {
-    acc = ld_xyzz(acc_io);
-    for (int d = 0; d < ndbl; d++) acc = coop_dbl(acc, role, base);
-    acc = coop_add(acc, v, role, base);
-  }
-  if (threadIdx.x == 0) st_xyzz(acc_io, acc);
-}
-__global__ void __launch_bounds__(32) k_finish(const XYZZ* __restrict__ acc_in, Affine* __restrict__ out, XYZZ* __restrict__ out_xyzz) {
-  if (threadIdx.x != 0) return;
-  XYZZ acc = ld_xyzz(acc_in);
-  if (out_xyzz) st_xyzz(out_xyzz, acc);
-  if (out) st_affine(out, xyzz_to_affine(acc, true));
-}
-
 // one QUAD per msm: Horner over windows (c doublings each), then canonical affine (optionally XYZZ partials for sharding)
-// pair = 1: a unit's window sum arrives as two addends, winsum[2u] + winsum[2u + 1] (column and row side of the 2-D bucket
-// reduction, k_pre_total)
 __global__ void __launch_bounds__(128) k_combine(const XYZZ* __restrict__ winsum, MsmShape sh, size_t nmsm, Affine* __restrict__ out,
-                                                 XYZZ* __restrict__ out_xyzz, int pair = 0) {
+                                                 XYZZ* __restrict__ out_xyzz) {
   size_t m = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 2;
   const int lane = threadIdx.x & 31, role = lane & 3, base = lane & ~3;
   const bool active = m < nmsm;
   if (!active) m = nmsm - 1;
-  const int np = pair ? 2 : 1;
-  const XYZZ* ws = winsum + m * sh.U * np;
-  XYZZ acc = ld_xyzz(ws + (size_t)(sh.U - 1) * np);
-#pragma unroll 1
-  for (int k = 1; k < np * (1 + sh.dbl); k++) {                                            // second addend / both units of the top window
-    XYZZ v = ld_xyzz(ws + (size_t)(sh.U - 1 - k / np) * np + k % np);
-    acc = coop_add(acc, v, role, base);
-  }
+  const XYZZ* ws = winsum + m * sh.U;
+  XYZZ acc = ld_xyzz(ws + sh.U - 1);
+  if (sh.dbl) { XYZZ v = ld_xyzz(ws + sh.U - 2); acc = coop_add(acc, v, role, base); }     // both units of the top window
   for (int w = sh.W - 2; w >= 0; w--) {
     for (int d = 0; d < sh.c; d++) acc = coop_dbl(acc, role, base);
-#pragma unroll 1
-    for (int k = 0; k < np; k++) { XYZZ v = ld_xyzz(ws + (size_t)w * np + k); acc = coop_add(acc, v, role, base); }
+    XYZZ v = ld_xyzz(ws + w);
+    acc = coop_add(acc, v, role, base);
   }
   if (!active || role != 0) return;
   if (out_xyzz) st_xyzz(out_xyzz + m, acc);
@@ -729,32 +688,29 @@ BP_DI Fq pre_load_scalar(const Fq* __restrict__ scalars, u32 t) {
   Fq k; k.v[0] = a.x; k.v[1] = a.y; k.v[2] = a.z; k.v[3] = a.w; k.v[4] = b.x; k.v[5] = b.y; k.v[6] = b.z; k.v[7] = b.w;
   return fq_reduce(k);                                  // es = [ei % order]   pippenger.py:26
 }
-// One thread per term: k mod q -> W signed digits of the windows of `ps`, histogram over the single bucket unit.  digits is [W][T]
-// (null: the scatter pass derives the digits again from the scalar -- 32 bytes read instead of 4 W written and read back).
-__global__ void __launch_bounds__(256) k_digits_pre(const Fq* __restrict__ scalars, u32 T, PreShape ps, int* __restrict__ digits,
-                                                    u32* __restrict__ bucket_count) {
+// One thread per term: k mod q -> W signed digits of the windows of `ps`, histogram over the single bucket unit.  No digit array:
+// the scatter pass derives the digits again from the scalar (32 bytes read instead of 4 W written and read back).
+__global__ void __launch_bounds__(256) k_digits_pre(const Fq* __restrict__ scalars, u32 T, PreShape ps, u32* __restrict__ bucket_count) {
   const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= T) return;
   const Fq k = pre_load_scalar(scalars, t);
   u32 carry = 0;
   for (int w = 0; w < ps.W; w++) {
     const int sd = pre_digit(k, ps, w, carry);
-    if (digits) digits[(size_t)w * T + t] = sd;
     if (sd != 0) atomicAdd(bucket_count + ((sd < 0 ? (u32)(-sd) : (u32)sd) - 1u), 1u);
   }
 }
 
 // counting-sort scatter: entry = {point index | sign << 31, bucket}, point index = w * stride + first + t
-__global__ void __launch_bounds__(256) k_scatter_pre(const int* __restrict__ digits, const Fq* __restrict__ scalars, u32 T, PreShape ps, u32 stride, u32 first,
+__global__ void __launch_bounds__(256) k_scatter_pre(const Fq* __restrict__ scalars, u32 T, PreShape ps, u32 stride, u32 first,
                                                      u32* __restrict__ cursor, uint2* __restrict__ entries, const u32* __restrict__ run_if = nullptr) {
   const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= T) return;
   if (run_if && __ldg(run_if) == 0) return;             // fallback of the slot sort: runs only when a bucket overflowed its slots
-  Fq k;
-  if (!digits) k = pre_load_scalar(scalars, t);
+  const Fq k = pre_load_scalar(scalars, t);
   u32 carry = 0;
   for (int w = 0; w < ps.W; w++) {
-    const int sd = digits ? digits[(size_t)w * T + t] : pre_digit(k, ps, w, carry);
+    const int sd = pre_digit(k, ps, w, carry);
     if (sd == 0) continue;
     const u32 bkt = (sd < 0 ? (u32)(-sd) : (u32)sd) - 1u;
     const u32 pos = atomicAdd(cursor + bkt, 1u);        // cursor[] starts at bucket_start[]: absolute slot
@@ -858,15 +814,9 @@ __global__ void __launch_bounds__(128, BP_ACC_MINB) k_accumulate_slots(const Aff
 // One launch reduces rows and columns by a factor K each (blockIdx.y = 0: rows, contiguous; 1: columns, strided):
 //   rows: out[i] = sum_{k<K} in[i*K + k]           (i < nrow_out)
 //   cols: out[g*C + lo] = sum_{k<K} in[(g*K + k)*C + lo]   (g < ncol_groups, lo < C)
-// blockIdx.z = bucket unit (plain path: the U units of an MSM are reduced side by side; `H` buckets apart on the input side, one
-// unit's worth of partial sums apart on the output side)
 __global__ void __launch_bounds__(128) k_pre_marginals(const XYZZ* __restrict__ row_in, XYZZ* __restrict__ row_out, u32 nrow_out, u32 Krow,
-                                                       const XYZZ* __restrict__ col_in, XYZZ* __restrict__ col_out, u32 ncol_groups, u32 C, u32 Kcol,
-                                                       u32 H = 0) {
+                                                       const XYZZ* __restrict__ col_in, XYZZ* __restrict__ col_out, u32 ncol_groups, u32 C, u32 Kcol) {
   const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
-  const size_t unit = blockIdx.z;
-  row_in += unit * H; col_in += unit * H;
-  row_out += unit * nrow_out; col_out += unit * ((size_t)ncol_groups * C);
   if (blockIdx.y == 0) {
     if (i >= nrow_out || Krow == 0) return;
     const XYZZ* src = row_in + (size_t)i * Krow;
@@ -888,13 +838,9 @@ __global__ void __launch_bounds__(128) k_pre_marginals(const XYZZ* __restrict__ 
 // C .. C+R-1: row hi, weight hi).  4-lane cooperative operations throughout (coop4.cuh: ~2 us per addition against ~4-8 us for
 // a lone thread's out-of-line call): the quads add the marginal's np partial sums (np <= 128, a power of two), a shared-memory
 // tree joins them, the first quad multiplies by the <= 11-bit weight (double-and-add) and stores wsum[block].
-// blockIdx.y = bucket unit; unit u with U > 0, dbl and u % U == U - 1 is the second unit of an MSM's top window, whose bucket
-// weights continue at H: its row weights are hi + R.
 __global__ void __launch_bounds__(64) k_pre_rowcol(const XYZZ* __restrict__ rowpart, u32 np_r, const XYZZ* __restrict__ colpart, u32 np_c,
-                                                   u32 C, u32 R, XYZZ* __restrict__ wsum, u32 U = 0, int dbl = 0) {
+                                                   u32 C, u32 R, XYZZ* __restrict__ wsum) {
   __shared__ XYZZ sm[16];
-  const size_t unit = blockIdx.y;
-  rowpart += unit * ((size_t)R * np_r); colpart += unit * ((size_t)np_c * C); wsum += unit * (C + R);
   const u32 bq = blockIdx.x, t = threadIdx.x, q = t >> 2;
   const int lane = t & 31, role = lane & 3, base = lane & ~3;
   const bool is_col = bq < C;
@@ -916,7 +862,7 @@ __global__ void __launch_bounds__(64) k_pre_rowcol(const XYZZ* __restrict__ rowp
   }
   if (t >= 32) return;                                   // the first warp (quad 0 holds the sum; its other quads shadow it)
   acc = sm[0];
-  const u32 wgt = is_col ? j + 1 : j + ((dbl && U && unit % U == U - 1) ? R : 0u);
+  const u32 wgt = is_col ? j + 1 : j;
   XYZZ r = xyzz_identity();
   for (int bit = 31 - __clz(wgt | 1u); bit >= 0; bit--) {
     r = coop_dbl(r, role, base);
@@ -926,11 +872,8 @@ __global__ void __launch_bounds__(64) k_pre_rowcol(const XYZZ* __restrict__ rowp
   if (t == 0) st_xyzz(wsum + bq, r);
 }
 // sums[side] = sum of wsum[side == 0 ? 0 .. C : C .. C+R): one block of 256 threads = 64 quads per side
-// blockIdx.y = bucket unit; ndbl > 0: the row side is multiplied by 2^ndbl here (plain path: C = 2^ndbl, the two sums of a unit
-// then simply add up to its window sum in k_combine's pair mode)
-__global__ void __launch_bounds__(256) k_pre_total(const XYZZ* __restrict__ wsum, u32 C, u32 R, XYZZ* __restrict__ sums, int ndbl = 0) {
+__global__ void __launch_bounds__(256) k_pre_total(const XYZZ* __restrict__ wsum, u32 C, u32 R, XYZZ* __restrict__ sums) {
   __shared__ XYZZ sm[64];
-  wsum += (size_t)blockIdx.y * (C + R); sums += 2 * (size_t)blockIdx.y;
   const u32 side = blockIdx.x, t = threadIdx.x, q = t >> 2, n = side == 0 ? C : R;
   const int lane = t & 31, role = lane & 3, base = lane & ~3;
   const XYZZ* src = wsum + (side == 0 ? 0u : C);
@@ -949,10 +892,6 @@ __global__ void __launch_bounds__(256) k_pre_total(const XYZZ* __restrict__ wsum
     if (q < off && role == 0) sm[q] = acc;
     __syncthreads();
   }
-  if (side == 1 && ndbl > 0 && t < 32) {                  // first warp: quad 0 holds the sum, the other quads shadow it
-    acc = sm[0];
-    for (int d = 0; d < ndbl; d++) acc = coop_dbl(acc, role, base);
-  }
   if (t == 0) st_xyzz(sums + side, acc);
 }
 // result = sums[0] + 2^lgC * sums[1]  (sums[0] = weighted columns, sums[1] = weighted rows); one quad
@@ -968,5 +907,3 @@ __global__ void __launch_bounds__(32) k_pre_finish(const XYZZ* __restrict__ sums
 }
 
 }  // namespace bp
-
-#include "affine.cuh"

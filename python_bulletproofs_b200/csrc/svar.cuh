@@ -57,12 +57,34 @@ __global__ void __launch_bounds__(128) k_rp_check_points(const Affine* __restric
   if (!affine_on_curve(ld_affine(pts + t))) bad[t / npt] = 1;
 }
 
+// Montgomery's trick across a warp: every lane receives the inverse of its own `acc` (all non-zero mod p) -- two shuffle scans
+// and ONE binary-GCD inversion by lane 31, which runs on the ALU pipe while the other warps of the SM keep the multiplier busy
+BP_DI Fp warp_batch_inverse(const Fp& acc, u32 lane) {
+  Fp S = acc, T = acc;                       // inclusive prefix / suffix products over the lanes
+#pragma unroll 1
+  for (int off = 1; off < 32; off <<= 1) {
+    const Fp a = shfl_up_fp(S, off), b = shfl_down_fp(T, off);
+    const bool up = lane >= (u32)off;        // S <- S * S[lane - off]   else   T <- T * T[lane + off]: both scans share one multiplier site
+    const Fp x = fp_mul(S, a);
+    const Fp y = fp_mul(T, b);
+    if (up) S = x;
+    if (lane + (u32)off < 32u) T = y;
+  }
+  Fp inv = fp_zero();
+  if (lane == 31) inv = fp_inv_gcd(S);       // 1 / (product of all 32)
+  inv = shfl_fp(inv, 31);
+  Fp Sm = shfl_up_fp(S, 1), Tp = shfl_down_fp(T, 1);
+  if (lane == 0) Sm = fp_one();
+  if (lane == 31) Tp = fp_one();
+  return fp_mul(fp_mul(Sm, Tp), inv);        // 1/acc_l = (acc_0 .. acc_{l-1}) * (acc_{l+1} .. acc_31) / total
+}
+
 // One thread per (proof, point slot).  pts = the chunk's proof points (npt per proof), vsc = its variable scalars (nv per proof,
 // written by k_rp_expand).  bad[] must be zeroed beforehand.  var_e3[p] receives -u_new (the whole variable part of E3).
 // The multiples 2P .. 8P leave the kernel in AFFINE form (T: 64 bytes per entry), so that k_sv_main's ~1300 additions per proof
 // are mixed additions (8M + 2S instead of 12M + 2S): the chain is built in XYZZ (parked in `scr`, with the prefix products of the
 // ZZZ values in `pre`), the product of a thread's seven ZZZ is inverted together with those of the 31 other lanes
-// (warp_batch_inverse, affine.cuh: two shuffle scans, one binary GCD per warp) and the thread walks back through its entries
+// (warp_batch_inverse above: two shuffle scans, one binary GCD per warp) and the thread walks back through its entries
 // (Montgomery's trick).  No thread leaves before the shared inversion; threads without a table contribute 1.
 __global__ void __launch_bounds__(128) k_sv_table(const Affine* __restrict__ pts, RpLayout lay, u32 cn, const Fq* __restrict__ vsc,
                                                   Affine* __restrict__ T, XYZZ* scr, Fp* pre, uint4* __restrict__ kd, u32* __restrict__ kflags,

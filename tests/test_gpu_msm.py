@@ -84,14 +84,14 @@ def test_msm_large_vs_oracle(lgn):
 
 @pytest.mark.parametrize("n", [(1 << 17), (1 << 17) + 3, 300001])
 def test_host_operand_msm_in_two_halves(n):
-    """bp_msm with >= 2^17 host terms uploads the points in two halves and accumulates the first while the second is on
-    the wire (msm_run, halves): same result as the device-resident path and the oracle, odd sizes and hot buckets included."""
+    """bp_msm with >= 2^17 host terms uploads its operands in parts and sorts and accumulates each part while the next is on
+    the wire (msm_run_parts): same result as the device-resident path and the oracle, odd sizes and hot buckets included."""
     base = fast_points(1 << 10, 777)
     rng = random.Random(n)
     pb = b"".join(ecc.pack_point(base[rng.randrange(len(base))]) for _ in range(n))
     ks = [rng.getrandbits(256) for _ in range(n)]
     for i in range(0, n, 7):
-        ks[i] = (1, 0, Q - 1, 2 ** 128, 5)[(i // 7) % 5]           # many equal scalars: giant buckets in both halves
+        ks[i] = (1, 0, Q - 1, 2 ** 128, 5)[(i // 7) % 5]           # many equal scalars: giant buckets in every part
     sb = b"".join(k.to_bytes(32, "little") for k in ks)
     got = gpu_msm_raw(pb, sb, n)
     assert got == ecc.msm_bytes(pb, sb, n, "bucket", ecc.max_threads())
@@ -201,9 +201,9 @@ def test_pippenger_dropin_api():
     assert P[0] + (-P[0]) == Point.IDENTITY_ELEMENT
 
 
-def test_device_resident_handles_and_pipelined_path():
-    """DevicePoints / DeviceScalars through Pippenger.multiexp, and the stream-pipelined single-MSM path
-    (off by default) must return the same point as the sequential path."""
+def test_device_resident_handles_and_forced_windows():
+    """DevicePoints / DeviceScalars through Pippenger.multiexp, with the automatic and with forced windows, must return the
+    oracle's point."""
     from python_bulletproofs_b200.pippenger import PipSECP256k1
     from python_bulletproofs_b200.device import DevicePoints, DeviceScalars
     from python_bulletproofs_b200 import Point, secp256k1
@@ -220,16 +220,12 @@ def test_device_resident_handles_and_pipelined_path():
     assert (r.x, r.y) == want
     lib = nat.load()
     try:
-        nat.check(lib.bp_msm_set_pipeline_min(1))
-        r = PipSECP256k1.multiexp(dp, ds)
-        assert (r.x, r.y) == want
         for c in (8, 13, 16):
             nat.check(lib.bp_msm_set_window(c))
             r = PipSECP256k1.multiexp(dp, ds)
             assert (r.x, r.y) == want, c
     finally:
         lib.bp_msm_set_window(0)
-        lib.bp_msm_set_pipeline_min(0)
     dp.free(); ds.free()
 
 
@@ -285,17 +281,16 @@ def test_msm_precomputed_window_multiples(c):
     dp.free()
 
 
-@pytest.mark.parametrize("passes", [1, 2, 3, 5])
+@pytest.mark.parametrize("kind", ["few_values", "pairs_cancel", "uniform", "sparse", "small"])
 @pytest.mark.parametrize("c", [8, 11])
-def test_msm_batched_affine_pair_passes(c, passes):
-    """affine.cuh: the pairwise affine passes ahead of the XYZZ accumulation (bp_msm_set_affine_passes), forced on a small
-    vector so that every special case sits in the pair sums: repeated points with equal scalars (P + P in one bucket), P and -P
-    (sum = identity, then identity + point in the next pass), identity inputs, all-equal scalars (one deep bucket per window),
-    zero scalars (empty buckets, padding only) -- against the oracle."""
+def test_msm_precomputed_deep_and_cancelling_buckets(c, kind):
+    """Precomputed path on a small vector whose buckets stress the XYZZ accumulation: repeated points with equal scalars (P + P
+    in one bucket), P and -P neighbours (sums that cancel to the identity, then identity + point), identity inputs, few distinct
+    or all-equal scalars (one deep bucket per window), zero scalars (empty buckets) -- full length and prefixes, against the oracle."""
     from python_bulletproofs_b200.device import DevicePoints
     n = 2500
     pool = fast_points(12, 777)
-    rng = random.Random(1000 * c + passes)
+    rng = random.Random(1000 * c)
     pts = [pool[rng.randrange(12)] for _ in range(n)]                 # 12 distinct points: most pairs inside a bucket are P + P
     for i in range(0, n, 7):
         pts[i] = ecc.point_neg(pts[i - 1]) if i else pts[i]           # P, -P neighbours
@@ -311,17 +306,13 @@ def test_msm_batched_affine_pair_passes(c, passes):
         "sparse": [0 if i % 5 else rng.getrandbits(256) for i in range(n)],
         "small": [rng.randrange(0, 4) for _ in range(n)],
     }
-    try:
-        nat.check(lib.bp_msm_set_affine_passes(passes))
-        for name, ks in scalar_sets.items():
-            sb = b"".join(int(k % 2 ** 256).to_bytes(32, "little") for k in ks)
-            nat.check(lib.bp_msm_h(dp.handle, sb, n, out))
-            assert ecc.unpack_point(out.raw) == ecc.msm(pts, [k % Q for k in ks]), name
-            for m in (1, 2, 31, 1025):
-                nat.check(lib.bp_msm_h(dp.handle, sb, m, out))
-                assert ecc.unpack_point(out.raw) == ecc.msm(pts[:m], [k % Q for k in ks[:m]]), (name, m)
-    finally:
-        lib.bp_msm_set_affine_passes(-1)
+    ks = scalar_sets[kind]
+    sb = b"".join(int(k % 2 ** 256).to_bytes(32, "little") for k in ks)
+    nat.check(lib.bp_msm_h(dp.handle, sb, n, out))
+    assert ecc.unpack_point(out.raw) == ecc.msm(pts, [k % Q for k in ks])
+    for m in (1, 2, 31, 1025):
+        nat.check(lib.bp_msm_h(dp.handle, sb, m, out))
+        assert ecc.unpack_point(out.raw) == ecc.msm(pts[:m], [k % Q for k in ks[:m]]), m
     dp.free()
 
 
@@ -343,10 +334,10 @@ def test_msm_precomputed_2p18_vs_plain_and_oracle():
     dp.free(); ds.free()
 
 
-def test_msm_experiment_switches_keep_the_result():
-    """bp_msm_set_tails2d (2-D marginal bucket reduction of the plain path's nine wide units, k_combine pair mode) and
-    bp_msm_set_chunk_fit (wave-fitted entries per accumulation thread, any chunk length): both measured slower and off by default,
-    both must give the bit-identical point -- resident operands (plain and precomputed) and host operands in parts."""
+def test_msm_2p18_resident_precomputed_host_parts_and_small_graph():
+    """One 2^18-term MSM four ways, each bit-identical to the oracle: resident operands on the plain path (nine wide bucket units)
+    and on the precomputed path, host operands (uploaded, sorted and accumulated in parts), and an odd-length prefix that takes
+    the precomputed vector's small-graph path."""
     n = 1 << 18
     from python_bulletproofs_b200.device import DevicePoints, DeviceScalars
     lib = nat.load()
@@ -356,17 +347,12 @@ def test_msm_experiment_switches_keep_the_result():
     want = ecc.pack_point(ecc.msm_bytes(base, sb, n, "bucket", ecc.max_threads()))
     dp, ds, dq = DevicePoints(raw=base), DeviceScalars(raw=sb), DevicePoints(raw=base).precompute(0)
     out = ctypes.create_string_buffer(64)
-    try:
-        for tails2d, fit in ((1, 0), (0, 1), (1, 1)):
-            nat.check(lib.bp_msm_set_tails2d(tails2d)); nat.check(lib.bp_msm_set_chunk_fit(fit))
-            nat.check(lib.bp_msm_hh(dp.handle, ds.handle, n, out)); assert out.raw == want, (tails2d, fit, "plain")
-            nat.check(lib.bp_msm_hh(dq.handle, ds.handle, n, out)); assert out.raw == want, (tails2d, fit, "pre")
-            nat.check(lib.bp_msm(base, sb, n, out)); assert out.raw == want, (tails2d, fit, "host operands")
-            m = (1 << 16) + 77                                        # small-graph path of the precomputed vector, odd length
-            nat.check(lib.bp_msm_hh(dq.handle, ds.handle, m, out))
-            assert out.raw == ecc.pack_point(ecc.msm_bytes(base, sb, m, "bucket", ecc.max_threads())), (tails2d, fit, m)
-    finally:
-        lib.bp_msm_set_tails2d(0); lib.bp_msm_set_chunk_fit(0)
+    nat.check(lib.bp_msm_hh(dp.handle, ds.handle, n, out)); assert out.raw == want, "plain"
+    nat.check(lib.bp_msm_hh(dq.handle, ds.handle, n, out)); assert out.raw == want, "pre"
+    nat.check(lib.bp_msm(base, sb, n, out)); assert out.raw == want, "host operands"
+    m = (1 << 16) + 77                                                # small-graph path of the precomputed vector, odd length
+    nat.check(lib.bp_msm_hh(dq.handle, ds.handle, m, out))
+    assert out.raw == ecc.pack_point(ecc.msm_bytes(base, sb, m, "bucket", ecc.max_threads())), m
     dp.free(); ds.free(); dq.free()
 
 

@@ -5,9 +5,7 @@ from python_bulletproofs_b200 import _native as nat
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 nat.init(0); lib = nat.load()
-lib.bp_msm_set_tails2d(int(os.environ.get("BP_TAILS2D", "0")))
 lib.bp_msm_set_host_finish(int(os.environ.get("BP_HOST_FINISH", "1")))
-lib.bp_msm_set_chunk_fit(int(os.environ.get("BP_CHUNK_FIT", "0")))
 lgn = int(sys.argv[1]) if len(sys.argv) > 1 else 20
 n = 1 << lgn
 pts, sc = bench.synth_inputs(n, 7)
@@ -17,5 +15,5 @@ ts = []
 for it in range(12):
     a = time.perf_counter(); nat.check(lib.bp_msm_sharded_host(pp, ps, n, out)); ts.append((time.perf_counter() - a) * 1e3)
 ts = sorted(ts[2:])
-print("e2e 2^%d: median %.3f ms best %.3f ms -> %.1f Mpts/s (piece %s MiB, split %s/8)" % (lgn, ts[len(ts) // 2], ts[0], n / ts[len(ts) // 2] / 1e3,
-      os.environ.get("BP_H2D_PIECE_MIB", "6"), os.environ.get("BP_E2E_SPLIT8", "3")), flush=True)
+print("e2e 2^%d: median %.3f ms best %.3f ms -> %.1f Mpts/s (piece %s MiB)" % (lgn, ts[len(ts) // 2], ts[0], n / ts[len(ts) // 2] / 1e3,
+      os.environ.get("BP_H2D_PIECE_MIB", "6")), flush=True)

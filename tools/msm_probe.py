@@ -32,10 +32,7 @@ def main():
     args = ap.parse_args()
     lib = nat.load()
     nat.init(0)
-    lib.bp_msm_set_tails2d(int(os.environ.get("BP_TAILS2D", "0")))
     lib.bp_msm_set_pre_slots(int(os.environ.get("BP_PRE_SLOTS", "1")), int(os.environ.get("BP_PRE_SLOTS_MIN", "0")))
-    lib.bp_msm_set_pre_fused(int(os.environ.get("BP_PRE_FUSED", "1")))
-    lib.bp_msm_set_chunk_fit(int(os.environ.get("BP_CHUNK_FIT", "0")))
     macs, ms = ctypes.c_double(), ctypes.c_float()
     nat.check(lib.bp_imad_peak(4096, ctypes.byref(macs), ctypes.byref(ms)))
     print("imad peak: %.3f T limb-MAC/s (%.2f ms)" % (macs.value / 1e12, ms.value), flush=True)
@@ -63,8 +60,6 @@ def main():
                 lgn, lib.bp_msm_last_window(), best, sorted(times)[len(times) // 2], n / best / 1e3)
                 + " ".join("%s=%.3f" % (nm, v) for nm, v in zip(names, stage)), flush=True)
     lib.bp_msm_set_window(0)
-    lib.bp_msm_set_pre_chunk(int(os.environ.get("BP_PRE_CHUNK", "0")))
-    lib.bp_msm_set_affine_passes(int(os.environ.get("BP_AFF_PASSES", "-1")))
     for pc in [int(x) for x in args.pre.split(",") if x != ""]:
         for lgn in [int(x) for x in args.lgn.split(",")]:
             n = 1 << lgn
