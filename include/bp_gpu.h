@@ -257,7 +257,9 @@ int bp_pipe_probe(int mode, int iters, double* ops_per_s, float* ms);
 
 /* ---- arithmetic self-test hooks (known-answer tests against big-int arithmetic) ------------------
  * fp: op 0 mul, 1 add, 2 sub, 3 inv, 4 neg  (inputs any 256-bit residue, output canonical)
- * ec: op 0 mixed add a+b, 1 full add, 2 double a, 3 negate a; +10 runs them on a re-projected a
+ * ec: op 0 mixed add a+b, 1 full add, 2 double a, 3 negate a; +10 runs them on a re-projected a;
+ *     op 4 coop_add(a, b), 5 coop_dbl(a): the 4-lane cooperative forms of csrc/coop4.cuh, one quad per pair (4n lanes, the last
+ *     warp padded with identity pairs); +10 re-projects both operands
  * fq: op 0 mul, 1 add, 2 sub, 3 inv, 4 neg; on_device = 0 runs the same code on the host; 5 mul, 6 inv, 7 square through
  *     the device-only standard-form arithmetic of csrc/fqdev.cuh (on_device = 0: the portable forms) */
 int bp_test_fp(int op, const uint8_t* a32, const uint8_t* b32, size_t n, uint8_t* out32);

@@ -116,6 +116,43 @@ def test_ec_ops_including_exceptional_cases():
     assert got == [ecc.point_neg(a) for a in A]
 
 
+def test_coop_ops_per_warp_case_mix():
+    """coop_add / coop_dbl (coop4.cuh), one quad per pair, 8 quads per warp.  The doubling pass runs for the whole warp when any
+    quad adds a point to itself, so the pairs are laid out warp by warp: all generic; one doubling quad (first, middle, last)
+    among generic ones; all doublings; doubling, opposite, O + b, a + O and O + O side by side; and a last, partial warp that
+    the kernel pads with identity pairs."""
+    rng = random.Random(44)
+    pool = [ecc.py_mul(ecc.G, rng.getrandbits(256)) for _ in range(40)]
+    pick = lambda: pool[rng.randrange(len(pool))]            # noqa: E731
+
+    def pair(kind):
+        a = pick()
+        if kind == "gen":
+            b = pick()
+            while b in (a, ecc.point_neg(a)):
+                b = pick()
+            return a, b
+        return {"dbl": (a, a), "opp": (a, ecc.point_neg(a)), "Ob": (None, a), "aO": (a, None), "OO": (None, None)}[kind]
+
+    warps = [["gen"] * 8] + [["gen"] * p + ["dbl"] + ["gen"] * (7 - p) for p in (0, 3, 7)] + [["dbl"] * 8]
+    warps += [["dbl", "opp", "Ob", "aO", "OO", "gen", "dbl", "opp"], ["opp", "gen", "OO", "dbl", "aO", "gen", "Ob", "opp"],
+              ["opp"] * 4 + ["Ob", "aO", "OO", "gen"], ["dbl", "Ob", "opp", "aO", "OO"]]
+    A, B = [], []
+    for w in warps:
+        for kind in w:
+            a, b = pair(kind)
+            A.append(a); B.append(b)
+    pa, pb, n = ecc.pack_points(A), ecc.pack_points(B), len(A)
+    assert n % 8 == 5
+    for op in (4, 14):
+        got = ecc.unpack_points(call_test("bp_test_ec", op, pa, pb, n, 64), n)
+        bad = [i for i in range(n) if got[i] != ecc.py_add(A[i], B[i])]
+        assert not bad, (op, [(i // 8, warps[i // 8][i % 8]) for i in bad])
+    for op in (5, 15):
+        got = ecc.unpack_points(call_test("bp_test_ec", op, pa, pb, n, 64), n)
+        assert got == [ecc.py_add(a, a) for a in A], op
+
+
 # ---- batched lift-x / decompression / generator derivation (SURVEY 8(f) N4) -------------------------------------
 def test_lift_x_batch_matches_big_int_square_roots():
     from python_bulletproofs_b200 import _native as nat

@@ -9,6 +9,7 @@ per proof.  Large batches are the pool's packed records tiled at the byte level,
 buffer, flag or verdict that leaks from one chunk into another then changes the decision pattern instead of repeating it."""
 import copy
 import ctypes
+import functools
 import os
 import pickle
 import random
@@ -120,11 +121,11 @@ def _pack(oVs, pr):
 class Pool:
     """D distinct proofs over one generator set: packed records, transcripts, start indices and the expected accept bytes."""
 
-    def __init__(self, n, m, D, tag, kind_shift=0):
+    def __init__(self, n, m, D, tag, kind_shift=0, generators=None):
         self.n, self.m, self.D = n, m, D
         nm = n * m
         self.L = nm.bit_length() - 1
-        self.ogs, self.ohs, self.og, self.oh, self.ou = gens(nm, [tag + "%d" % i for i in range(5)])
+        self.ogs, self.ohs, self.og, self.oh, self.ou = generators or gens(nm, [tag + "%d" % i for i in range(5)])
         self.gens = (self.og, self.oh, self.ogs, self.ohs, self.ou)          # argument order of verify_packed
         self.packed_gens = pack_generators(self.og, self.oh, self.ogs, self.ohs, self.ou)
         gs, hs, g, h, u = [P_(t) for t in self.ogs], [P_(t) for t in self.ohs], P_(self.og), P_(self.oh), P_(self.ou)
@@ -425,3 +426,37 @@ def test_knobs_read_once_per_process(tmp_path, pools):
     env.pop("LOCAL_WORLD_SIZE", None)
     out = subprocess.run([sys.executable, str(script), ROOT, str(data)], env=env, capture_output=True, text=True, timeout=600)
     assert out.returncode == 0 and out.stdout.strip().endswith("OK"), (out.stdout[-2000:], out.stderr[-4000:])
+
+
+# ---- a generator set whose own sums collide -------------------------------------------------------------------------------
+def _degenerate_generators(n, tag):
+    """gs = [P1, -P1, P2, -P2, ...] (Gsum = O), hs = [Q1, Q1, Q2, Q2, ...] (Hsum a sum of doublings), u = g."""
+    base = [po.elliptic_hash(b"%s%d" % (tag, i)) for i in range(n + 2)]
+    gs = [p for i in range(n // 2) for p in (base[i], _neg(base[i]))]
+    hs = [base[n // 2 + i // 2] for i in range(n)]
+    g, h = base[n], base[n + 1]
+    return gs, hs, g, h, g
+
+
+def test_degenerate_generator_set(fb_mode):
+    """The verifier's own sums of a generator set (k_sum_points: Gsum, Hsum) on a set where they cancel and double; every accept
+    byte against the oracle under table modes 0, 1 and 2, then the set alternated with an ordinary one of the same length in one
+    process, so that the Gsum / Hsum kept from one set can never serve the other."""
+    n = 16
+    gens16 = _degenerate_generators(n, b"degenerate")
+    assert functools.reduce(ecc.point_add, gens16[0]) is None
+    deg = Pool(n, 1, 64, "degenerate", generators=gens16)
+    plain = Pool(n, 1, 31, "ordinary16_")
+    deg_batch, deg_want, deg_kinds = deg.tile(64, 0)
+    plain_batch, plain_want, plain_kinds = plain.tile(93, 5)
+    for mode in (0, 1, 2):
+        fb_mode(mode)
+        for call in range(2):
+            _same(_verify(deg, deg_batch), deg_want, deg_kinds, "degenerate set, fb mode %d, call %d" % (mode, call))
+    for mode in (0, 1):
+        fb_mode(mode)
+        for step in range(6):
+            if step % 2:
+                _same(_verify(plain, plain_batch), plain_want, plain_kinds, "ordinary set, fb mode %d, step %d" % (mode, step))
+            else:
+                _same(_verify(deg, deg_batch), deg_want, deg_kinds, "degenerate set, fb mode %d, step %d" % (mode, step))
