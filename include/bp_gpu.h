@@ -228,6 +228,22 @@ size_t bp_rp_aggreg_proof_stride(size_t n, size_t m);
 int bp_rp_verify_aggreg_batch(const uint8_t* gs64, const uint8_t* hs64, const uint8_t g64[64], const uint8_t h64[64], const uint8_t u64_[64],
                               size_t n, size_t m, const uint8_t* proofs, size_t proof_stride, size_t nproofs, const uint8_t* transcripts,
                               const uint64_t* tr_off, const uint32_t* start_transcript, uint8_t* accept);
+/* Batch verification by ONE random linear combination (csrc/bp_rlc.inl, csrc/rlc.cuh).  Inputs as for bp_rp_verify_aggreg_batch
+ * (m = 1: the record of bp_rp_verify_batch, byte for byte).  Proof p's equations E1..E4 are weighted with rho_p^1..rho_p^4,
+ * rho_p = SHA-256(seed32 || le64(p)) read little-endian, mod q (1 if that is 0), and summed; the sum is tested once.
+ * A proof whose transcript checks give 0 or 2, or with a point off the curve / not canonical (accept byte 0), stays out of the sum.
+ *   sum == identity: every proof in it is accepted, *combined = 1 (also for an empty batch or one in which no proof entered);
+ *   otherwise:       *combined = 0 and accept holds the bytes of the exact verifier over the whole batch (bp_rp_verify_batch for
+ *                    m = 1 and n <= 128, else bp_rp_verify_aggreg_batch).
+ * Guarantee: the decisions equal the exact verifier's except with probability <= 4/q, PROVIDED seed32 is unpredictable to whoever
+ * made the proofs -- draw it from a CSPRNG for every call.  A fixed or guessable seed lets an adversary craft invalid proofs whose
+ * errors cancel in the sum (two proofs off by d and -d rho_0/rho_1 are then both accepted); the parameter exists for
+ * reproducibility and tests.  seed32 = NULL is an error; so are a bad n*m, a short proof_stride and nproofs*(m + 6 + 2 log2(n m))
+ * >= 2^31.  combined may be NULL. */
+int bp_rp_verify_batch_rlc(const uint8_t* gs64, const uint8_t* hs64, const uint8_t g64[64], const uint8_t h64[64], const uint8_t u64_[64],
+                           size_t n, size_t m, const uint8_t* proofs, size_t proof_stride, size_t nproofs, const uint8_t* transcripts,
+                           const uint64_t* tr_off, const uint32_t* start_transcript, const uint8_t seed32[32],
+                           uint8_t* accept, int* combined);
 /* measurements of the last batch call: [0] wall ms, [1] host transcript-check ms (sum over chunks), [2] device span ms
  * (CUDA events on the library stream: first chunk's first kernel .. last accept kernel), [3] chunks, [4] host threads,
  * [5] table mode (0 bucket method, 1 byte tables, 2 16-bit tables), [6] proofs */

@@ -19,6 +19,7 @@
 #include "svar.cuh"
 #include "fixedbase.cuh"
 #include "ipa_round.cuh"
+#include "rlc.cuh"
 #include "rp_algebra.h"
 #include <nccl.h>
 #include <thread>
@@ -1027,3 +1028,4 @@ int bp_imad_peak(int iters, double* macs_per_s, float* ms_out) { BP_NEED_INIT();
 }  // extern "C"
 #include "bp_proto.inl"
 #include "bp_aggreg.inl"
+#include "bp_rlc.inl"

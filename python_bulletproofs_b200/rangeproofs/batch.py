@@ -6,6 +6,7 @@ Packing of a proof follows include/bp_gpu.h (bp_rp_verify_batch); the per-proof 
 checks run in C on host threads, the scalar algebra and all point equations on the GPU.
 """
 import ctypes
+import os
 
 from .. import _native as nat
 from .rangeproof_verifier import RangeVerifier
@@ -113,14 +114,15 @@ def verify_stats():
             "table_mode": int(v[5]), "proofs": int(v[6])}
 
 
-def verify_range_proofs_batch(Vs, g, h, gs, hs, u, proofs):
+def verify_range_proofs_batch(Vs, g, h, gs, hs, u, proofs, combine=False, seed=None):
     """-> list[bool].  A proof the C layer cannot classify (exotic numeric transcript slot) is replayed
-    through RangeVerifier so that the reference's exception type (ValueError / IndexError) surfaces."""
+    through RangeVerifier so that the reference's exception type (ValueError / IndexError) surfaces.
+    combine=True checks one random linear combination of the whole batch first (verify_rlc_packed; seed as there)."""
     n = len(gs)
     if len(Vs) != len(proofs):
         raise Exception('Different number of commitments and proofs')
     batch = PackedBatch.from_proofs(Vs, proofs, n)
-    acc = verify_packed(batch, g, h, gs, hs, u)
+    acc = verify_rlc_packed(batch, g, h, gs, hs, u, seed)[0] if combine else verify_packed(batch, g, h, gs, hs, u)
     out = []
     for i, a in enumerate(acc):
         if a == 2:
@@ -196,10 +198,31 @@ def verify_aggreg_packed(batch: PackedAggregBatch, g, h, gs, hs, u, packed=None)
     return accept.raw[:batch.nproofs]
 
 
-def verify_aggreg_range_proofs_batch(Vs_list, g, h, gs, hs, u, proofs):
+def verify_rlc_packed(batch, g, h, gs, hs, u, seed=None, packed=None):
+    """-> (accept bytes, combined) of a PackedBatch (m = 1) or PackedAggregBatch through bp_rp_verify_batch_rlc: one random
+    linear combination of every proof's equations is checked; combined = 1 when it holds (every proof that passed its
+    transcript and point checks is accepted), 0 when it does not (the bytes are then the exact verifier's).
+    seed=None draws 32 fresh bytes from os.urandom for this call.  The decisions are the exact verifier's except with
+    probability <= 4/q only while the seed is unknown to whoever made the proofs: pass a fixed seed for reproducible tests,
+    never for proofs from an untrusted source."""
+    if seed is None:
+        seed = os.urandom(32)
+    if len(seed) != 32:
+        raise ValueError("seed must be 32 bytes")
+    accept = ctypes.create_string_buffer(max(batch.nproofs, 1))
+    combined = ctypes.c_int(0)
+    gs_b, hs_b, g_b, h_b, u_b = packed if packed is not None else pack_generators(g, h, gs, hs, u)
+    nat.check(nat.load().bp_rp_verify_batch_rlc(gs_b, hs_b, g_b, h_b, u_b, batch.n, getattr(batch, "m", 1), batch.records,
+                                                batch.stride, batch.nproofs, batch.blob, batch.tr_off, batch.starts, bytes(seed),
+                                                accept, ctypes.byref(combined)))
+    return accept.raw[:batch.nproofs], combined.value
+
+
+def verify_aggreg_range_proofs_batch(Vs_list, g, h, gs, hs, u, proofs, combine=False, seed=None):
     """-> list[bool]: AggregRangeVerifier(Vs_i, g, h, gs, hs, u, proof_i).verify() for every i, in one call
     (rangeproof_aggreg_verifier.py:42-108).  A proof the C layer cannot classify is replayed through AggregRangeVerifier so that
-    the reference's exception type surfaces."""
+    the reference's exception type surfaces.  combine=True checks one random linear combination of the whole batch first
+    (verify_rlc_packed; seed as there)."""
     from .rangeproof_aggreg_verifier import AggregRangeVerifier
     if len(Vs_list) != len(proofs):
         raise Exception('Different number of commitments and proofs')
@@ -209,7 +232,7 @@ def verify_aggreg_range_proofs_batch(Vs_list, g, h, gs, hs, u, proofs):
     if len(gs) % m:
         raise ValueError("generator count is not a multiple of the number of commitments")
     batch = PackedAggregBatch.from_proofs(Vs_list, proofs, len(gs) // m)
-    acc = verify_aggreg_packed(batch, g, h, gs, hs, u)
+    acc = verify_rlc_packed(batch, g, h, gs, hs, u, seed)[0] if combine else verify_aggreg_packed(batch, g, h, gs, hs, u)
     out = []
     for i, a in enumerate(acc):
         if a == 2:
