@@ -244,6 +244,25 @@ int bp_rp_verify_batch_rlc(const uint8_t* gs64, const uint8_t* hs64, const uint8
                            size_t n, size_t m, const uint8_t* proofs, size_t proof_stride, size_t nproofs, const uint8_t* transcripts,
                            const uint64_t* tr_off, const uint32_t* start_transcript, const uint8_t seed32[32],
                            uint8_t* accept, int* combined);
+/* One random linear combination over a batch of MIXED shapes (csrc/bp_rlc.inl): proof p has n = ns[p] bits per value and
+ * m = ms[p] values, N_p = ns[p]*ms[p] a power of two <= nset, and is checked against the prefixes gs[:N_p], hs[:N_p] of one set of
+ * nset <= 2048 generators per side (gs64, hs64: nset points each) -- AggregRangeVerifier(Vs_p, g, h, gs[:N_p], hs[:N_p], u,
+ * proof_p).verify(), with m = 1 RangeVerifier.  Records back to back in the caller's order, each bp_rp_aggreg_proof_stride(ns[p],
+ * ms[p]) bytes (m = 1: the bp_rp_verify_batch record), proofs_bytes their sum; transcripts / tr_off / start_transcript and the
+ * accept bytes as for bp_rp_verify_batch_rlc.  Weights rho_p as there, p the index in the caller's order; one sum over every proof
+ * of every shape, tested once (all shapes' generator columns add into the 2 nset + 5 rows of the set, whose byte table is the one
+ * bp_rp_verify_aggreg_batch / bp_rp_verify_batch_rlc build for n*m = nset).
+ *   sum == identity: every proof in it is accepted, *combined = 1 (also for an empty batch);
+ *   otherwise:       *combined = 0 and each shape is decided by the exact verifier over its prefix set (bp_rp_verify_batch for
+ *                    m = 1 and n <= 128, else bp_rp_verify_aggreg_batch), the bytes in the caller's order.
+ * Guarantee as for bp_rp_verify_batch_rlc: the decisions equal the exact verifier's except with probability <= 4/q, PROVIDED
+ * seed32 is unpredictable to whoever made the proofs -- draw it from a CSPRNG for every call.  Errors: seed32 = NULL, nset > 2048,
+ * a shape with N_p not a power of two or larger than nset, proofs_bytes not the sum of the record sizes, and
+ * sum_p (m_p + 6 + 2 log2 N_p) >= 2^31.  combined may be NULL. */
+int bp_rp_verify_mixed_rlc(const uint8_t* gs64, const uint8_t* hs64, const uint8_t g64[64], const uint8_t h64[64], const uint8_t u64_[64],
+                           size_t nset, const uint32_t* ns, const uint32_t* ms, const uint8_t* proofs, size_t proofs_bytes,
+                           size_t nproofs, const uint8_t* transcripts, const uint64_t* tr_off, const uint32_t* start_transcript,
+                           const uint8_t seed32[32], uint8_t* accept, int* combined);
 /* measurements of the last batch call: [0] wall ms, [1] host transcript-check ms (sum over chunks), [2] device span ms
  * (CUDA events on the library stream: first chunk's first kernel .. last accept kernel), [3] chunks, [4] host threads,
  * [5] table mode (0 bucket method, 1 byte tables, 2 16-bit tables), [6] proofs */

@@ -9,6 +9,7 @@
 #include <mutex>
 #include <string>
 #include <vector>
+#include <algorithm>
 
 #include "../../include/bp_gpu.h"
 #include "ctx.h"

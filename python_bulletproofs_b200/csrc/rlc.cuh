@@ -8,7 +8,8 @@
 //                       | L_j -w4 x_j^2 | R_j -w4 x_j^-2
 // k_rlc_prep (a warp per proof) gathers and curve-checks the proof's points, writes their scalars and a small table per proof;
 // k_rlc_fold adds the tables' products into the 2N generator columns (a thread per column pair, proofs of a group from shared
-// memory); k_rlc_colsum adds the groups in a fixed order (mod-q sums, no atomics: the result does not depend on scheduling).
+// memory); k_rlc_colsum adds the groups in a fixed order (mod-q sums, no atomics: the result does not depend on scheduling) into
+// the 2 nset + 5 columns of the generator set, of which a proof of N <= nset generators per side uses the prefixes gs[:N], hs[:N].
 // Standard-form arithmetic of fqdev.cuh throughout.
 #pragma once
 #include "verify.cuh"
@@ -188,7 +189,9 @@ __global__ void __launch_bounds__(128) k_rlc_prep(const uint8_t* __restrict__ re
 
 // part[grp][0, N) = gs columns, [N, 2N) = hs columns, [2N, 2N+5) = g, h, u, Gsum, Hsum of the G proofs of group grp.  A thread
 // owns generator position i (its gs and its hs column): per proof 1 + 4 multiplications, sums in registers.
-__global__ void __launch_bounds__(128) k_rlc_fold(const Fq* __restrict__ tabs, RlcShape s, u32 cn, u32 G, Fq* __restrict__ part) {
+// spread != 0 (proofs shorter than the set, N < nset): the set's Gsum / Hsum rows sum more generators than the proof uses, so
+// each proof's -w2 z and w2 z go into its own N gs / hs columns instead and the Gsum / Hsum entries of part are 0.
+__global__ void __launch_bounds__(128) k_rlc_fold(const Fq* __restrict__ tabs, RlcShape s, u32 cn, u32 G, u32 spread, Fq* __restrict__ part) {
   extern __shared__ Fq smt[];
   const u32 grp = blockIdx.y, p0 = grp * G, np = cn - p0 < G ? cn - p0 : G;
   {
@@ -212,24 +215,31 @@ __global__ void __launch_bounds__(128) k_rlc_fold(const Fq* __restrict__ tabs, R
       accG = fq_add(accG, fq_mul_dev(ld_fq(T + ih), ld_fq(T + oB + il)));                                   // w4 a s_i
       const Fq v = fq_add(fq_mul_dev(ld_fq(T + oG), t2k), fq_mul_dev(ld_fq(T + H + chi), ld_fq(T + oB + clo)));  // w2 z^(2+j) 2^k + w4 b s_{N-1-i}
       accH = fq_add(accH, fq_mul_dev(fq_mul_dev(ld_fq(T + oAy + ih), ld_fq(T + oBy + il)), v));               // times y^-i
+      if (spread) {
+        accG = fq_add(accG, ld_fq(T + rlc_oCol(s) + 3));                                                   // -w2 z
+        accH = fq_add(accH, ld_fq(T + rlc_oCol(s) + 4));                                                   // w2 z
+      }
     }
     st_fq(out + i, accG);
     st_fq(out + s.N + i, accH);
   }
   if (blockIdx.x == 0 && threadIdx.x < 5) {
     Fq acc = fq_zero();
-    for (u32 q = 0; q < np; q++) acc = fq_add(acc, ld_fq(smt + (size_t)q * s.ts + rlc_oCol(s) + threadIdx.x));
+    if (!spread || threadIdx.x < 3)
+      for (u32 q = 0; q < np; q++) acc = fq_add(acc, ld_fq(smt + (size_t)q * s.ts + rlc_oCol(s) + threadIdx.x));
     st_fq(out + 2 * s.N + threadIdx.x, acc);
   }
 }
 
-// col[c] += sum over the groups of part[grp][c], groups in order
-__global__ void __launch_bounds__(128) k_rlc_colsum(const Fq* __restrict__ part, u32 ngroups, u32 F, Fq* __restrict__ col) {
-  const u32 c = blockIdx.x * blockDim.x + threadIdx.x;
+// col[set column of c] += sum over the groups of part[grp][c], groups in order.  part has the 2N + 5 columns of a proof of N
+// generators per side, col the 2 nset + 5 of the set: gs_i stays at i, hs_i goes to nset + i, the five tail columns to 2 nset + k.
+__global__ void __launch_bounds__(128) k_rlc_colsum(const Fq* __restrict__ part, u32 ngroups, u32 N, u32 nset, Fq* __restrict__ col) {
+  const u32 F = 2 * N + 5, c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= F) return;
-  Fq acc = ld_fq(col + c);
+  const u32 dst = c < N ? c : c < 2 * N ? nset + (c - N) : 2 * nset + (c - 2 * N);
+  Fq acc = ld_fq(col + dst);
   for (u32 k = 0; k < ngroups; k++) acc = fq_add(acc, ld_fq(part + (size_t)k * F + c));
-  st_fq(col + c, acc);
+  st_fq(col + dst, acc);
 }
 
 // out[0] = 1 if the XYZZ partials (one per chunk, then the generator MSM) add up to the identity

@@ -24,6 +24,17 @@ def pack_proof(V, proof, log_n):
     return b"".join(rec), (proof.transcript, ip.transcript, p2.transcript), p2.start_transcript
 
 
+def pack_transcripts(transcripts, starts):
+    """-> (blob, tr_off, starts) of the C ABI: every proof's three transcripts in one blob with 3 * nproofs + 1 offsets."""
+    offs, blob, pos = [0], [], 0
+    for trio in transcripts:
+        for t in trio:
+            blob.append(t)
+            pos += len(t)
+            offs.append(pos)
+    return b"".join(blob), (ctypes.c_uint64 * len(offs))(*offs), (ctypes.c_uint32 * max(len(starts), 1))(*starts)
+
+
 class PackedBatch:
     """A batch in the wire layout of bp_rp_verify_batch (struct-of-records + transcript blob)."""
 
@@ -32,15 +43,7 @@ class PackedBatch:
         self.nproofs = len(records)
         self.records = b"".join(records)
         self.stride = len(records[0]) if records else nat.load().bp_rp_proof_stride(n)
-        offs, blob, pos = [0], [], 0
-        for trio in transcripts:
-            for t in trio:
-                blob.append(t)
-                pos += len(t)
-                offs.append(pos)
-        self.blob = b"".join(blob)
-        self.tr_off = (ctypes.c_uint64 * len(offs))(*offs)
-        self.starts = (ctypes.c_uint32 * max(len(starts), 1))(*starts)
+        self.blob, self.tr_off, self.starts = pack_transcripts(transcripts, starts)
 
     @classmethod
     def from_proofs(cls, Vs, proofs, n):
@@ -240,6 +243,98 @@ def verify_aggreg_range_proofs_batch(Vs_list, g, h, gs, hs, u, proofs, combine=F
             try:
                 with contextlib.redirect_stdout(io.StringIO()):
                     out.append(bool(AggregRangeVerifier(Vs_list[i], g, h, gs, hs, u, proofs[i]).verify()))
+            except Exception as e:   # noqa: BLE001
+                if str(e) == "Proof invalid":
+                    out.append(False)
+                else:
+                    raise
+        else:
+            out.append(a == 1)
+    return out
+
+
+# ---- proofs of mixed shapes over prefixes of one generator set ----------------------------------------------------------------
+class PackedMixedBatch:
+    """A batch in the wire layout of bp_rp_verify_mixed_rlc: proofs of any shape (n bits, m values; n * m a power of two <= nset)
+    over the prefixes gs[:n*m], hs[:n*m] of one set of nset generators per side, records back to back in the caller's order."""
+
+    def __init__(self, nset, ns, ms, records, transcripts, starts):
+        self.nset = nset
+        self.nproofs = len(records)
+        self.ns, self.ms = list(ns), list(ms)
+        self.offsets, pos = [], 0                  # byte offset of every record
+        for r in records:
+            self.offsets.append(pos)
+            pos += len(r)
+        self.records = b"".join(records)
+        self.blob, self.tr_off, self.starts = pack_transcripts(transcripts, starts)
+        self.ns_arr = (ctypes.c_uint32 * max(len(ns), 1))(*ns)
+        self.ms_arr = (ctypes.c_uint32 * max(len(ms), 1))(*ms)
+
+    @classmethod
+    def from_items(cls, items, nset):
+        """items: (V, proof) or (Vs, proof) pairs; a bare V is a single-value proof (m = 1), a list Vs an aggregated one of m =
+        len(Vs) values.  The proof's length N = 2^len(xs) gives n = N / m."""
+        ns, ms, recs, trs, sts = [], [], [], [], []
+        for V, pr in items:
+            Vs = V if isinstance(V, list) else [V]
+            p2 = pr.innerProof.proof2
+            m, L = len(Vs), len(p2.xs)
+            N = 1 << L
+            if m == 0 or N % m or len(p2.Ls) != L or len(p2.Rs) != L:
+                raise ValueError("proof shape does not match its number of commitments")
+            if N > nset:
+                raise ValueError("proof of %d generators per side is larger than the set of %d" % (N, nset))
+            r, t, s = pack_aggreg_proof(Vs, pr, L)
+            if any(not (0 <= int(getattr(x, "x", x)) < nat.Q) for x in p2.xs):      # unreduced challenge: step-by-step path (see PackedBatch)
+                s = 0xFFFFFFFF
+            ns.append(N // m)
+            ms.append(m)
+            recs.append(r)
+            trs.append(t)
+            sts.append(s)
+        return cls(nset, ns, ms, recs, trs, sts)
+
+
+def verify_mixed_rlc_packed(batch: PackedMixedBatch, g, h, gs, hs, u, seed=None, packed=None):
+    """-> (accept bytes, combined) of a PackedMixedBatch through bp_rp_verify_mixed_rlc: one random linear combination of every
+    proof's equations, whatever its shape; combined = 1 when it holds, 0 when it does not (the bytes are then the exact
+    verifiers', one call per shape).  gs, hs: the set of batch.nset generators per side (packed = pack_generators(...) of it).
+    seed as for verify_rlc_packed: None draws 32 fresh bytes from os.urandom; a fixed seed only for reproducible tests."""
+    if seed is None:
+        seed = os.urandom(32)
+    if len(seed) != 32:
+        raise ValueError("seed must be 32 bytes")
+    gs_b, hs_b, g_b, h_b, u_b = packed if packed is not None else pack_generators(g, h, gs, hs, u)
+    if len(gs_b) != 64 * batch.nset or len(hs_b) != 64 * batch.nset:
+        raise ValueError("the batch was packed for a set of %d generators per side" % batch.nset)
+    accept = ctypes.create_string_buffer(max(batch.nproofs, 1))
+    combined = ctypes.c_int(0)
+    nat.check(nat.load().bp_rp_verify_mixed_rlc(gs_b, hs_b, g_b, h_b, u_b, batch.nset, batch.ns_arr, batch.ms_arr, batch.records,
+                                                len(batch.records), batch.nproofs, batch.blob, batch.tr_off, batch.starts, bytes(seed),
+                                                accept, ctypes.byref(combined)))
+    return accept.raw[:batch.nproofs], combined.value
+
+
+def verify_mixed_range_proofs_batch(items, g, h, gs, hs, u, seed=None):
+    """-> list[bool] in the order of `items`, (V, proof) or (Vs, proof) pairs of any shape over prefixes of one generator set:
+    RangeVerifier(V, g, h, gs[:N], hs[:N], u, proof).verify() for a bare V, AggregRangeVerifier(Vs, ...) for a list, N = n * m
+    the proof's length -- in one call (one random linear combination, seed as for verify_rlc_packed).  A proof the C layer cannot
+    classify is replayed through those classes so that the reference's exception type surfaces.  ValueError: a proof larger than
+    the set."""
+    from .rangeproof_aggreg_verifier import AggregRangeVerifier
+    batch = PackedMixedBatch.from_items(items, len(gs))
+    acc = verify_mixed_rlc_packed(batch, g, h, gs, hs, u, seed)[0]
+    out = []
+    for i, a in enumerate(acc):
+        if a == 2:
+            import contextlib, io
+            V, pr = items[i]
+            N = batch.ns[i] * batch.ms[i]
+            cls = AggregRangeVerifier if isinstance(V, list) else RangeVerifier
+            try:
+                with contextlib.redirect_stdout(io.StringIO()):
+                    out.append(bool(cls(V, g, h, gs[:N], hs[:N], u, pr).verify()))
             except Exception as e:   # noqa: BLE001
                 if str(e) == "Proof invalid":
                     out.append(False)
