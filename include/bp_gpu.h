@@ -263,6 +263,30 @@ int bp_rp_verify_mixed_rlc(const uint8_t* gs64, const uint8_t* hs64, const uint8
                            size_t nset, const uint32_t* ns, const uint32_t* ms, const uint8_t* proofs, size_t proofs_bytes,
                            size_t nproofs, const uint8_t* transcripts, const uint64_t* tr_off, const uint32_t* start_transcript,
                            const uint8_t seed32[32], uint8_t* accept, int* combined);
+/* The random linear combination of bp_rp_verify_mixed_rlc, and when it fails, the invalid proofs LOCATED by sub-combinations
+ * instead of the exact verifier over the whole batch (csrc/bp_rlc.inl, csrc/rlc.cuh).  Arguments as for bp_rp_verify_mixed_rlc
+ * (a batch of one shape passes ns[p] = n, ms[p] = m for every p and nset = n*m), plus `leaf`.
+ *   sum == identity: the result of bp_rp_verify_mixed_rlc, *combined = 1; no leaf work runs.
+ *   otherwise:       *combined = 0.  The batch, in the order it is processed (grouped by shape, cut into chunks of 64 .. 2048
+ *                    proofs of one shape), is cut into leaves of `leaf` consecutive proofs of one chunk (the last leaf of a chunk
+ *                    may be shorter).  Each leaf's part of the weighted sum is tested on the device; the proofs of failing leaves
+ *                    that entered the sum are decided by the exact verifier of their shape (bp_rp_verify_batch for m = 1 and
+ *                    n <= 128, else bp_rp_verify_aggreg_batch), the others keep the byte of the combination (1).
+ * Proofs settled before the sum (transcript verdict 0 or 2, a point off the curve or not canonical) keep that byte, which is the
+ * exact verifier's.  leaf = 0 lets the library pick (the smallest power of two >= sqrt(512 nproofs^2 / sum_p n_p m_p), within
+ * 8 .. 256); an explicit leaf places the boundaries for tests and is not a performance switch.
+ * Guarantee: a rejection is exact.  When the whole sum fails, at least one leaf fails (the leaf sums add up to it).  The accept
+ * bytes equal the exact verifier's except with probability <= 4 (K + 1)/q for K leaves, PROVIDED seed32 is unpredictable to whoever
+ * made the proofs (as for bp_rp_verify_batch_rlc).  Errors: those of bp_rp_verify_mixed_rlc, leaf >= 2^32, and a leaf pass larger
+ * than its 32-bit offsets (K (2 nset + 5) >= 2^30).  combined may be NULL. */
+int bp_rp_verify_rlc_locate(const uint8_t* gs64, const uint8_t* hs64, const uint8_t g64[64], const uint8_t h64[64], const uint8_t u64_[64],
+                            size_t nset, const uint32_t* ns, const uint32_t* ms, const uint8_t* proofs, size_t proofs_bytes,
+                            size_t nproofs, const uint8_t* transcripts, const uint64_t* tr_off, const uint32_t* start_transcript,
+                            const uint8_t seed32[32], size_t leaf, uint8_t* accept, int* combined);
+/* the last bp_rp_verify_rlc_locate call: [0] leaf size used, [1] leaves (0: no leaf pass ran), [2] failing leaves, [3] proofs
+ * of failing leaves that entered the sum, i.e. decided by the exact step (when every leaf fails, the exact verifier runs over the
+ * whole batch as in bp_rp_verify_mixed_rlc; the settled proofs keep the bytes they had) */
+int bp_rp_rlc_locate_stats(uint64_t out4[4]);
 /* measurements of the last batch call: [0] wall ms, [1] host transcript-check ms (sum over chunks), [2] device span ms
  * (CUDA events on the library stream: first chunk's first kernel .. last accept kernel), [3] chunks, [4] host threads,
  * [5] table mode (0 bucket method, 1 byte tables, 2 16-bit tables), [6] proofs */

@@ -81,6 +81,10 @@ PROTOTYPES = {
     "bp_rp_verify_mixed_rlc": (ctypes.c_int, [c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_sz, ctypes.POINTER(ctypes.c_uint32),
                                               ctypes.POINTER(ctypes.c_uint32), c_u8p, c_sz, c_sz, c_u8p, ctypes.POINTER(ctypes.c_uint64),
                                               ctypes.POINTER(ctypes.c_uint32), c_u8p, c_u8p, ctypes.POINTER(ctypes.c_int)]),
+    "bp_rp_verify_rlc_locate": (ctypes.c_int, [c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_sz, ctypes.POINTER(ctypes.c_uint32),
+                                               ctypes.POINTER(ctypes.c_uint32), c_u8p, c_sz, c_sz, c_u8p, ctypes.POINTER(ctypes.c_uint64),
+                                               ctypes.POINTER(ctypes.c_uint32), c_u8p, c_sz, c_u8p, ctypes.POINTER(ctypes.c_int)]),
+    "bp_rp_rlc_locate_stats": (ctypes.c_int, [ctypes.POINTER(ctypes.c_uint64)]),
     "bp_mod_hash": (ctypes.c_int, [c_u8p, c_sz, c_u8p]),
     "bp_mod_hash_indexed": (ctypes.c_int, [c_u8p, c_sz, ctypes.c_uint32, ctypes.c_uint32, c_u8p]),
     "bp_sha256": (ctypes.c_int, [c_u8p, c_sz, c_u8p]),

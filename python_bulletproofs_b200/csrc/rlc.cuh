@@ -250,4 +250,37 @@ __global__ void k_rlc_final(const XYZZ* __restrict__ parts, u32 nparts, uint8_t*
   out[0] = xyzz_is_identity(acc) ? 1 : 0;
 }
 
+// Leaf pass of bp_rp_verify_rlc_locate (bp_rlc.inl): a leaf is a run of consecutive proofs of one chunk made of whole fold groups,
+// leaf[k] = {offset of its first group's partials in part, its groups, N of its shape}.  A thread per (leaf k, set column c):
+// cols[k F + c] = the leaf's partials of the part column that k_rlc_colsum maps to c, groups in order (fixed order, no atomics);
+// offs[k] = k F (the leaves' generator MSMs end to end, F = 2 nset + 5); rows[k F + c] = c (the generator row of every term).
+__global__ void __launch_bounds__(128) k_rlc_leaf_cols(const Fq* __restrict__ part, const uint4* __restrict__ leaf, u32 K, u32 nset,
+                                                       Fq* __restrict__ cols, u32* __restrict__ offs, u32* __restrict__ rows) {
+  const u32 F = 2 * nset + 5;
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (size_t)K * F) return;
+  const u32 k = (u32)(t / F), c = (u32)(t - (size_t)k * F);
+  const uint4 d = leaf[k];
+  const u32 N = d.z, FN = 2 * N + 5;
+  const u32 pc = c < nset ? (c < N ? c : FN) : c < 2 * nset ? (c - nset < N ? N + (c - nset) : FN) : 2 * N + (c - 2 * nset);
+  Fq acc = fq_zero();
+  if (pc < FN)
+    for (u32 q = 0; q < d.y; q++) acc = fq_add(acc, ld_fq(part + d.x + (size_t)q * FN + pc));
+  st_fq(cols + t, acc);
+  rows[t] = c;
+  if (c == 0) offs[k] = k * F;
+  if (t == 0) offs[K] = K * F;
+}
+
+// out[k] = 1 if leaf k's generator part and proof-point part add up to the identity
+__global__ void __launch_bounds__(128) k_rlc_leaf_test(const XYZZ* __restrict__ gen, const XYZZ* __restrict__ pts, u32 K,
+                                                       uint8_t* __restrict__ out) {
+  const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= K) return;
+  XYZZ a = ld_xyzz(gen + k);
+  const XYZZ b = ld_xyzz(pts + k);
+  xyzz_add_ni(a, b);
+  out[k] = xyzz_is_identity(a) ? 1 : 0;
+}
+
 }  // namespace bp

@@ -5,6 +5,7 @@
 Packing of a proof follows include/bp_gpu.h (bp_rp_verify_batch); the per-proof transcript
 checks run in C on host threads, the scalar algebra and all point equations on the GPU.
 """
+import array
 import ctypes
 import os
 
@@ -117,15 +118,20 @@ def verify_stats():
             "table_mode": int(v[5]), "proofs": int(v[6])}
 
 
-def verify_range_proofs_batch(Vs, g, h, gs, hs, u, proofs, combine=False, seed=None):
+def verify_range_proofs_batch(Vs, g, h, gs, hs, u, proofs, combine=False, seed=None, locate=False):
     """-> list[bool].  A proof the C layer cannot classify (exotic numeric transcript slot) is replayed
     through RangeVerifier so that the reference's exception type (ValueError / IndexError) surfaces.
-    combine=True checks one random linear combination of the whole batch first (verify_rlc_packed; seed as there)."""
+    combine=True checks one random linear combination of the whole batch first (verify_rlc_packed; seed as there).
+    locate=True implies it and, when it fails, sends only the proofs of failing leaves to the exact verifier
+    (verify_rlc_locate_packed)."""
     n = len(gs)
     if len(Vs) != len(proofs):
         raise Exception('Different number of commitments and proofs')
     batch = PackedBatch.from_proofs(Vs, proofs, n)
-    acc = verify_rlc_packed(batch, g, h, gs, hs, u, seed)[0] if combine else verify_packed(batch, g, h, gs, hs, u)
+    if locate:
+        acc = verify_rlc_locate_packed(batch, g, h, gs, hs, u, seed)[0]
+    else:
+        acc = verify_rlc_packed(batch, g, h, gs, hs, u, seed)[0] if combine else verify_packed(batch, g, h, gs, hs, u)
     out = []
     for i, a in enumerate(acc):
         if a == 2:
@@ -221,11 +227,12 @@ def verify_rlc_packed(batch, g, h, gs, hs, u, seed=None, packed=None):
     return accept.raw[:batch.nproofs], combined.value
 
 
-def verify_aggreg_range_proofs_batch(Vs_list, g, h, gs, hs, u, proofs, combine=False, seed=None):
+def verify_aggreg_range_proofs_batch(Vs_list, g, h, gs, hs, u, proofs, combine=False, seed=None, locate=False):
     """-> list[bool]: AggregRangeVerifier(Vs_i, g, h, gs, hs, u, proof_i).verify() for every i, in one call
     (rangeproof_aggreg_verifier.py:42-108).  A proof the C layer cannot classify is replayed through AggregRangeVerifier so that
     the reference's exception type surfaces.  combine=True checks one random linear combination of the whole batch first
-    (verify_rlc_packed; seed as there)."""
+    (verify_rlc_packed; seed as there).  locate=True implies it and, when it fails, sends only the proofs of failing leaves to
+    the exact verifier (verify_rlc_locate_packed)."""
     from .rangeproof_aggreg_verifier import AggregRangeVerifier
     if len(Vs_list) != len(proofs):
         raise Exception('Different number of commitments and proofs')
@@ -235,7 +242,10 @@ def verify_aggreg_range_proofs_batch(Vs_list, g, h, gs, hs, u, proofs, combine=F
     if len(gs) % m:
         raise ValueError("generator count is not a multiple of the number of commitments")
     batch = PackedAggregBatch.from_proofs(Vs_list, proofs, len(gs) // m)
-    acc = verify_rlc_packed(batch, g, h, gs, hs, u, seed)[0] if combine else verify_aggreg_packed(batch, g, h, gs, hs, u)
+    if locate:
+        acc = verify_rlc_locate_packed(batch, g, h, gs, hs, u, seed)[0]
+    else:
+        acc = verify_rlc_packed(batch, g, h, gs, hs, u, seed)[0] if combine else verify_aggreg_packed(batch, g, h, gs, hs, u)
     out = []
     for i, a in enumerate(acc):
         if a == 2:
@@ -316,15 +326,57 @@ def verify_mixed_rlc_packed(batch: PackedMixedBatch, g, h, gs, hs, u, seed=None,
     return accept.raw[:batch.nproofs], combined.value
 
 
-def verify_mixed_range_proofs_batch(items, g, h, gs, hs, u, seed=None):
+def verify_rlc_locate_packed(batch, g, h, gs, hs, u, seed=None, packed=None, leaf=0):
+    """-> (accept bytes, combined) of a PackedBatch, PackedAggregBatch or PackedMixedBatch through bp_rp_verify_rlc_locate: the
+    random linear combination of verify_rlc_packed / verify_mixed_rlc_packed (same weights, same result when it holds,
+    combined = 1); when it fails (combined = 0) the batch is cut into leaves of consecutive proofs, each leaf's part of the sum is
+    tested, and only the proofs of failing leaves go to the exact verifier.  leaf=0 lets the library pick the leaf size; an
+    explicit leaf places the boundaries (for tests).  The decisions are the exact verifier's except with probability
+    <= 4 (K + 1)/q for K leaves, only while the seed is unknown to whoever made the proofs: seed=None draws 32 fresh bytes from
+    os.urandom; pass a fixed seed for reproducible tests, never for proofs from an untrusted source."""
+    if seed is None:
+        seed = os.urandom(32)
+    if len(seed) != 32:
+        raise ValueError("seed must be 32 bytes")
+    if leaf < 0:
+        raise ValueError("leaf must be >= 0")
+    if isinstance(batch, PackedMixedBatch):
+        nset, ns_arr, ms_arr = batch.nset, batch.ns_arr, batch.ms_arr
+    else:
+        m = getattr(batch, "m", 1)
+        nset = batch.n * m
+        cnt = max(batch.nproofs, 1)
+        ns_arr = (ctypes.c_uint32 * cnt).from_buffer(array.array("I", [batch.n]) * cnt)
+        ms_arr = (ctypes.c_uint32 * cnt).from_buffer(array.array("I", [m]) * cnt)
+    gs_b, hs_b, g_b, h_b, u_b = packed if packed is not None else pack_generators(g, h, gs, hs, u)
+    if len(gs_b) != 64 * nset or len(hs_b) != 64 * nset:
+        raise ValueError("the batch was packed for a set of %d generators per side" % nset)
+    accept = ctypes.create_string_buffer(max(batch.nproofs, 1))
+    combined = ctypes.c_int(0)
+    nat.check(nat.load().bp_rp_verify_rlc_locate(gs_b, hs_b, g_b, h_b, u_b, nset, ns_arr, ms_arr, batch.records, len(batch.records),
+                                                 batch.nproofs, batch.blob, batch.tr_off, batch.starts, bytes(seed), leaf, accept,
+                                                 ctypes.byref(combined)))
+    return accept.raw[:batch.nproofs], combined.value
+
+
+def rlc_locate_stats():
+    """dict of the last verify_rlc_locate_packed call (bp_rp_rlc_locate_stats): leaf size used, leaves (0 when no leaf pass ran),
+    failing leaves, proofs decided by the exact verifier."""
+    v = (ctypes.c_uint64 * 4)()
+    nat.check(nat.load().bp_rp_rlc_locate_stats(v))
+    return {"leaf": v[0], "leaves": v[1], "failing_leaves": v[2], "exact_proofs": v[3]}
+
+
+def verify_mixed_range_proofs_batch(items, g, h, gs, hs, u, seed=None, locate=False):
     """-> list[bool] in the order of `items`, (V, proof) or (Vs, proof) pairs of any shape over prefixes of one generator set:
     RangeVerifier(V, g, h, gs[:N], hs[:N], u, proof).verify() for a bare V, AggregRangeVerifier(Vs, ...) for a list, N = n * m
     the proof's length -- in one call (one random linear combination, seed as for verify_rlc_packed).  A proof the C layer cannot
     classify is replayed through those classes so that the reference's exception type surfaces.  ValueError: a proof larger than
-    the set."""
+    the set.  locate=True: when the combination fails, only the proofs of failing leaves go to the exact verifier
+    (verify_rlc_locate_packed)."""
     from .rangeproof_aggreg_verifier import AggregRangeVerifier
     batch = PackedMixedBatch.from_items(items, len(gs))
-    acc = verify_mixed_rlc_packed(batch, g, h, gs, hs, u, seed)[0]
+    acc = (verify_rlc_locate_packed if locate else verify_mixed_rlc_packed)(batch, g, h, gs, hs, u, seed)[0]
     out = []
     for i, a in enumerate(acc):
         if a == 2:
