@@ -287,9 +287,24 @@ int bp_rp_verify_rlc_locate(const uint8_t* gs64, const uint8_t* hs64, const uint
  * of failing leaves that entered the sum, i.e. decided by the exact step (when every leaf fails, the exact verifier runs over the
  * whole batch as in bp_rp_verify_mixed_rlc; the settled proofs keep the bytes they had) */
 int bp_rp_rlc_locate_stats(uint64_t out4[4]);
-/* measurements of the last batch call: [0] wall ms, [1] host transcript-check ms (sum over chunks), [2] device span ms
- * (CUDA events on the library stream: first chunk's first kernel .. last accept kernel), [3] chunks, [4] host threads,
- * [5] table mode (0 bucket method, 1 byte tables, 2 16-bit tables), [6] proofs */
+/* Batch PROVER (csrc/bp_prove.inl): AggregNIRangeProver(vs_p, n, g, h, gs, hs, gammas_p, u, secp256k1, seed_p).prove() for every
+ * proof p (NIRangeProver when m = 1), byte for byte.  N = n*m a power of two <= 2048, gs64 / hs64 N points each.
+ * values32, gammas32: nproofs*m scalars (32 bytes little-endian), proof-major, taken as the reference takes v.x / gamma.x: the
+ * bits are (v >> i) & 1 for i < n (a value >= 2^n gives the same invalid proof as the per-proof prover), gamma is reduced mod q.
+ * seeds: the proofs' transcript seeds back to back, proof p's at [seed_off[p], seed_off[p+1]) (nproofs + 1 offsets).  The blinding
+ * factors derive from the seed alone, as in the reference: two proofs with the same seed share them.
+ * Output = the input of bp_rp_verify_aggreg_batch / bp_rp_verify_batch_rlc:
+ *   records: nproofs * bp_rp_aggreg_proof_stride(n, m) bytes, V_j = v_j g + gamma_j h first (m = 1: the bp_rp_verify_batch record);
+ *   transcripts / tr_off (3 nproofs + 1 offsets) / start_transcript: each proof's range, Protocol-1 and Protocol-2 transcripts.
+ * Errors: a bad n*m, and tr_cap smaller than the transcripts (*tr_len receives the bytes needed; records are complete).
+ * nproofs = 0 does no device work.  Measurements through bp_rp_verify_stats. */
+int bp_rp_prove_batch(const uint8_t* gs64, const uint8_t* hs64, const uint8_t g64[64], const uint8_t h64[64], const uint8_t u64_[64],
+                      size_t n, size_t m, const uint8_t* values32, const uint8_t* gammas32, const uint8_t* seeds,
+                      const uint64_t* seed_off, size_t nproofs, uint8_t* records, uint8_t* transcripts, size_t tr_cap,
+                      size_t* tr_len, uint64_t* tr_off, uint32_t* start_transcript);
+/* measurements of the last batch call, bp_rp_verify_batch or bp_rp_prove_batch: [0] wall ms, [1] host ms (transcript checks /
+ * prover host steps, sum over chunks), [2] device span ms (CUDA events on the library stream: first chunk's first kernel .. last
+ * kernel), [3] chunks, [4] host threads, [5] table mode (0 bucket method, 1 byte tables, 2 16-bit tables), [6] proofs */
 int bp_rp_verify_stats(double out7[7]);
 
 /* ---- host-side Fiat-Shamir helpers (exported for tests; src/utils/utils.py:84-111) -------------- */

@@ -85,6 +85,9 @@ PROTOTYPES = {
                                                ctypes.POINTER(ctypes.c_uint32), c_u8p, c_sz, c_sz, c_u8p, ctypes.POINTER(ctypes.c_uint64),
                                                ctypes.POINTER(ctypes.c_uint32), c_u8p, c_sz, c_u8p, ctypes.POINTER(ctypes.c_int)]),
     "bp_rp_rlc_locate_stats": (ctypes.c_int, [ctypes.POINTER(ctypes.c_uint64)]),
+    "bp_rp_prove_batch": (ctypes.c_int, [c_u8p, c_u8p, c_u8p, c_u8p, c_u8p, c_sz, c_sz, c_u8p, c_u8p, c_u8p,
+                                         ctypes.POINTER(ctypes.c_uint64), c_sz, c_u8p, c_u8p, c_sz, ctypes.POINTER(c_sz),
+                                         ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint32)]),
     "bp_mod_hash": (ctypes.c_int, [c_u8p, c_sz, c_u8p]),
     "bp_mod_hash_indexed": (ctypes.c_int, [c_u8p, c_sz, ctypes.c_uint32, ctypes.c_uint32, c_u8p]),
     "bp_sha256": (ctypes.c_int, [c_u8p, c_sz, c_u8p]),

@@ -1030,3 +1030,4 @@ int bp_imad_peak(int iters, double* macs_per_s, float* ms_out) { BP_NEED_INIT();
 #include "bp_proto.inl"
 #include "bp_aggreg.inl"
 #include "bp_rlc.inl"
+#include "bp_prove.inl"

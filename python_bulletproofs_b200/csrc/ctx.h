@@ -66,6 +66,7 @@ struct Ctx {
   // IPA / verifier workspaces
   DevBuf ws_g, ws_h, ws_a, ws_b, ws_g2, ws_h2, ws_a2, ws_b2, ws_idx, ws_lr, ws_terms_sc, ws_small;
   DevBuf ws_sv_tab, ws_sv_acc, ws_sv_sc, ws_rp_sums;      // batch verifier: variable-point tables / window sums / split scalars; Gsum, Hsum
+  DevBuf ws_prove;                                        // batch prover: generator rows, two chunks' state, term patterns
   std::vector<unsigned char> rp_sums_src; unsigned long long rp_sums_gen = 0;   // generator bytes the kept sums belong to
   cudaStream_t var_stream[2] = {nullptr, nullptr};        // batch verifier: proof-specific terms, concurrent with the table lookups (one per chunk parity,
                                                           // so that the doubling chains of consecutive chunks overlap)
@@ -188,7 +189,7 @@ struct Ctx {
     DevBuf* all[] = {&ws_pts, &ws_sc, &ws_off, &ws_out, &ws_digits, &ws_entries, &ws_count, &ws_start, &ws_cursor, &ws_tiles,
                      &ws_buckets, &ws_segsum, &ws_winsum, &ws_misc, &ws_flush, &ws_g, &ws_h, &ws_a, &ws_b, &ws_g2, &ws_h2,
                      &ws_a2, &ws_b2, &ws_idx, &ws_lr, &ws_terms_sc, &ws_small, &ws_entry_bucket, &ws_part, &ws_big, &ws_phi, &ws_segrun, &ws_grpsum, &ws_winpart, &ws_fb_lanes, &ws_fb_var, &ws_sv_tab, &ws_sv_acc, &ws_sv_sc, &ws_rp_sums,
-                     &ws_ipa_rp, &ws_ipa_ticket, &ws_slots, &ws_slots_ovf};
+                     &ws_ipa_rp, &ws_ipa_ticket, &ws_slots, &ws_slots_ovf, &ws_prove};
     rp_sums_src.clear();
     for (DevBuf* b : all) b->release();
   }

@@ -134,6 +134,41 @@ __global__ void __launch_bounds__(256) k_build_lr(const Fq* __restrict__ a, cons
 // are therefore two (n+1)-term multi-scalar multiplications over the original points with scalars a*cg / b*ch -- the
 // same group elements as the reference computes, at the cost of one batched MSM per round and no 256-bit scalar
 // multiplication per generator.  cg, ch are kept in Montgomery form; a, b in standard form.
+// Point numbering of the terms: g_t -> g0 + t, h_t -> h0 + t, u -> iu.  A single proof's points are [u | g (n) | h (n)]
+// = {1, 1 + n, 0}; a batch of range proofs addresses the rows of its generator set instead (bp_prove.inl).
+struct IpaRows { u32 g0, h0, iu; };
+
+// a'[t] = x*a[t] + xinv*a[m+t], b'[t] = xinv*b[t] + x*b[m+t] for t < m (inner_product_prover.py:109-110) and the coefficient
+// update cg[t] *= (upper ? x : x^-1), ch[t] *= (upper ? x^-1 : x) for the generator fold (:107-108); m = new length, 2m = old.
+BP_DI void ipa_fold_elem(Fq* __restrict__ a, Fq* __restrict__ b, Fq* __restrict__ cg, Fq* __restrict__ ch, u32 t, u32 m,
+                         const Fq& xm, const Fq& xim) {
+  const bool hi = (t % (2 * m)) >= m;
+  st_fq(cg + t, fq_mont(ld_fq(cg + t), hi ? xm : xim));
+  st_fq(ch + t, fq_mont(ld_fq(ch + t), hi ? xim : xm));
+  if (t < m) {
+    Fq alo = ld_fq(a + t), ahi = ld_fq(a + m + t), blo = ld_fq(b + t), bhi = ld_fq(b + m + t);
+    st_fq(a + t, fq_add(fq_mont(alo, xm), fq_mont(ahi, xim)));
+    st_fq(b + t, fq_add(fq_mont(blo, xim), fq_mont(bhi, xm)));
+  }
+}
+// The L and R terms of original generator t (t < n) in a round of length m: slots [0, n/2) g-part, [n/2, n) h-part of
+// each MSM, R at offset n + 1
+BP_DI void ipa_lr_term(const Fq* __restrict__ a, const Fq* __restrict__ b, const Fq* __restrict__ cg, const Fq* __restrict__ ch,
+                       u32 t, u32 n, u32 m, IpaRows rows, Fq* __restrict__ tsc, u32* __restrict__ tidx) {
+  const u32 k = m >> 1, n1 = n + 1;
+  const u32 i = t % m, blk = t / m;
+  const bool hi = i >= k;
+  const u32 slot = blk * k + (hi ? i - k : i);                 // position among the n/2 terms of its kind
+  const Fq cgt = ld_fq(cg + t), cht = ld_fq(ch + t);
+  if (hi) {
+    st_fq(tsc + slot, fq_mont(ld_fq(a + i - k), cgt));              tidx[slot] = rows.g0 + t;              // L: a_lo[i-k] * g_t
+    st_fq(tsc + n1 + n / 2 + slot, fq_mont(ld_fq(b + i - k), cht)); tidx[n1 + n / 2 + slot] = rows.h0 + t; // R: b_lo[i-k] * h_t
+  } else {
+    st_fq(tsc + n1 + slot, fq_mont(ld_fq(a + i + k), cgt));         tidx[n1 + slot] = rows.g0 + t;         // R: a_hi[i] * g_t
+    st_fq(tsc + n / 2 + slot, fq_mont(ld_fq(b + i + k), cht));      tidx[n / 2 + slot] = rows.h0 + t;      // L: b_hi[i] * h_t
+  }
+}
+
 // One block of 256 threads.  Points live in [u | g (n) | h (n)].
 __global__ void __launch_bounds__(256) k_build_lr_sv(const Fq* __restrict__ a, const Fq* __restrict__ b, const Fq* __restrict__ cg,
                                                      const Fq* __restrict__ ch, u32 n, const u32* __restrict__ m_ptr, Fq* __restrict__ tsc,
@@ -146,20 +181,7 @@ __global__ void __launch_bounds__(256) k_build_lr_sv(const Fq* __restrict__ a, c
     accl = fq_add(accl, fq_mont(ld_fq(a + i), ld_fq(b + k + i)));
     accr = fq_add(accr, fq_mont(ld_fq(a + k + i), ld_fq(b + i)));
   }
-  // L terms: slots [0, n/2) g-part, [n/2, n) h-part, n = u ;  R terms follow at offset n1
-  for (u32 t = threadIdx.x; t < n; t += 256) {
-    const u32 i = t % m, blk = t / m;
-    const bool hi = i >= k;
-    const u32 slot = blk * k + (hi ? i - k : i);               // position among the n/2 terms of its kind
-    const Fq cgt = ld_fq(cg + t), cht = ld_fq(ch + t);
-    if (hi) {
-      tsc[slot] = fq_mont(ld_fq(a + i - k), cgt);              tidx[slot] = 1 + t;                       // L: a_lo[i-k] * g_t
-      tsc[n1 + n / 2 + slot] = fq_mont(ld_fq(b + i - k), cht); tidx[n1 + n / 2 + slot] = 1 + n + t;      // R: b_lo[i-k] * h_t
-    } else {
-      tsc[n1 + slot] = fq_mont(ld_fq(a + i + k), cgt);         tidx[n1 + slot] = 1 + t;                  // R: a_hi[i] * g_t
-      tsc[n / 2 + slot] = fq_mont(ld_fq(b + i + k), cht);      tidx[n / 2 + slot] = 1 + n + t;           // L: b_hi[i] * h_t
-    }
-  }
+  for (u32 t = threadIdx.x; t < n; t += 256) ipa_lr_term(a, b, cg, ch, t, n, m, IpaRows{1, 1 + n, 0}, tsc, tidx);
   sl[threadIdx.x] = accl; sr[threadIdx.x] = accr;
   __syncthreads();
   for (int off = 128; off > 0; off >>= 1) {
@@ -195,66 +217,32 @@ struct IpaRound {
 __global__ void __launch_bounds__(128) k_round_fold(Fq* __restrict__ a, Fq* __restrict__ b, Fq* __restrict__ cg, Fq* __restrict__ ch, u32 n,
                                                     const IpaRound* __restrict__ rp) {
   if (!rp->fold) return;
-  const u32 t = blockIdx.x * blockDim.x + threadIdx.x, m = rp->m;
+  const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= n) return;
-  const Fq xm = ld_fq(&rp->xm), xim = ld_fq(&rp->xim);
-  const bool hi = (t % (2 * m)) >= m;
-  st_fq(cg + t, fq_mont(ld_fq(cg + t), hi ? xm : xim));
-  st_fq(ch + t, fq_mont(ld_fq(ch + t), hi ? xim : xm));
-  if (t < m) {
-    Fq alo = ld_fq(a + t), ahi = ld_fq(a + m + t), blo = ld_fq(b + t), bhi = ld_fq(b + m + t);
-    st_fq(a + t, fq_add(fq_mont(alo, xm), fq_mont(ahi, xim)));
-    st_fq(b + t, fq_add(fq_mont(blo, xim), fq_mont(bhi, xm)));
-  }
+  ipa_fold_elem(a, b, cg, ch, t, rp->m, ld_fq(&rp->xm), ld_fq(&rp->xim));
 }
-// One round's scalar work in ONE block (n <= 4096; the latency-bound small proofs): k_round_fold, a block barrier, then
-// k_build_lr_sv (build = 1) or, after the last challenge, the copy-out of the final a, b (build = 0, ab_out may be mapped host
-// memory).  rp may live in mapped host memory too: it is read once into shared memory.
-__global__ void __launch_bounds__(1024) k_ipa_round_prep(Fq* __restrict__ a, Fq* __restrict__ b, Fq* __restrict__ cg, Fq* __restrict__ ch, u32 n,
-                                                         const IpaRound* __restrict__ rp, Fq* __restrict__ tsc, u32* __restrict__ tidx,
-                                                         int build, Fq* __restrict__ ab_out) {
-  __shared__ IpaRound s_rp;
+// One round's scalar work of one proof in ONE block: the fold with the previous challenge (fold), a block barrier, then the L/R
+// terms with c_L, c_R (build = 1) or, after the last challenge, the copy-out of the final a, b (build = 0).  The u terms get
+// c * umul R^-2: umul = R^2 gives c itself, x R^2 gives x c (terms over u when the proof's generator is u_new = x u).
+BP_DI void ipa_round_block(Fq* __restrict__ a, Fq* __restrict__ b, Fq* __restrict__ cg, Fq* __restrict__ ch, u32 n, u32 m, bool fold,
+                           const Fq& xm, const Fq& xim, int build, IpaRows rows, const Fq& umul, Fq* __restrict__ tsc,
+                           u32* __restrict__ tidx, Fq* __restrict__ ab_out) {
   __shared__ Fq sl[32], sr[32];
-  if (threadIdx.x < sizeof(IpaRound) / 4) ((u32*)&s_rp)[threadIdx.x] = ((const volatile u32*)rp)[threadIdx.x];
-  __syncthreads();
-  const u32 m = s_rp.m;
-  if (s_rp.fold) {                                             // (k_round_fold) m = new length, 2m = old length
-    const Fq xm = s_rp.xm, xim = s_rp.xim;
-    for (u32 t = threadIdx.x; t < n; t += blockDim.x) {
-      const bool hi = (t % (2 * m)) >= m;
-      st_fq(cg + t, fq_mont(ld_fq(cg + t), hi ? xm : xim));
-      st_fq(ch + t, fq_mont(ld_fq(ch + t), hi ? xim : xm));
-      if (t < m) {
-        Fq alo = ld_fq(a + t), ahi = ld_fq(a + m + t), blo = ld_fq(b + t), bhi = ld_fq(b + m + t);
-        st_fq(a + t, fq_add(fq_mont(alo, xm), fq_mont(ahi, xim)));
-        st_fq(b + t, fq_add(fq_mont(blo, xim), fq_mont(bhi, xm)));
-      }
-    }
+  if (fold) {
+    for (u32 t = threadIdx.x; t < n; t += blockDim.x) ipa_fold_elem(a, b, cg, ch, t, m, xm, xim);
     __syncthreads();                                           // the folded a, b, cg, ch are visible to the whole block
   }
   if (!build) {
     if (threadIdx.x == 0) { st_fq(ab_out, ld_fq(a)); st_fq(ab_out + 1, ld_fq(b)); __threadfence_system(); }
     return;
   }
-  const u32 k = m >> 1, n1 = n + 1;                             // (k_build_lr_sv)
+  const u32 k = m >> 1, n1 = n + 1;
   Fq accl = fq_zero(), accr = fq_zero();
   for (u32 i = threadIdx.x; i < k; i += blockDim.x) {
     accl = fq_add(accl, fq_mont(ld_fq(a + i), ld_fq(b + k + i)));
     accr = fq_add(accr, fq_mont(ld_fq(a + k + i), ld_fq(b + i)));
   }
-  for (u32 t = threadIdx.x; t < n; t += blockDim.x) {
-    const u32 i = t % m, blk = t / m;
-    const bool hi = i >= k;
-    const u32 slot = blk * k + (hi ? i - k : i);
-    const Fq cgt = ld_fq(cg + t), cht = ld_fq(ch + t);
-    if (hi) {
-      st_fq(tsc + slot, fq_mont(ld_fq(a + i - k), cgt));              tidx[slot] = 1 + t;
-      st_fq(tsc + n1 + n / 2 + slot, fq_mont(ld_fq(b + i - k), cht)); tidx[n1 + n / 2 + slot] = 1 + n + t;
-    } else {
-      st_fq(tsc + n1 + slot, fq_mont(ld_fq(a + i + k), cgt));         tidx[n1 + slot] = 1 + t;
-      st_fq(tsc + n / 2 + slot, fq_mont(ld_fq(b + i + k), cht));      tidx[n / 2 + slot] = 1 + n + t;
-    }
-  }
+  for (u32 t = threadIdx.x; t < n; t += blockDim.x) ipa_lr_term(a, b, cg, ch, t, n, m, rows, tsc, tidx);
   // inner products: lane sums by shuffles, warp sums through shared memory
   const u32 lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
   for (int off = 16; off > 0; off >>= 1) {
@@ -274,10 +262,32 @@ __global__ void __launch_bounds__(1024) k_ipa_round_prep(Fq* __restrict__ a, Fq*
       accl = fq_add(accl, xl); accr = fq_add(accr, xr);
     }
     if (lane == 0) {
-      st_fq(tsc + n, fq_to_mont(accl));       tidx[n] = 0;             // (sum * R^-1) * R ; point u
-      st_fq(tsc + n1 + n, fq_to_mont(accr));  tidx[n1 + n] = 0;
+      st_fq(tsc + n, fq_mont(accl, umul));       tidx[n] = rows.iu;        // (sum * R^-1) * umul * R^-1 ; point u
+      st_fq(tsc + n1 + n, fq_mont(accr, umul));  tidx[n1 + n] = rows.iu;
     }
   }
+}
+// The latency-bound small proofs (n <= 4096): one round of one proof per launch.  rp and ab_out may live in mapped host
+// memory: rp is read once into shared memory.
+__global__ void __launch_bounds__(1024) k_ipa_round_prep(Fq* __restrict__ a, Fq* __restrict__ b, Fq* __restrict__ cg, Fq* __restrict__ ch, u32 n,
+                                                         const IpaRound* __restrict__ rp, Fq* __restrict__ tsc, u32* __restrict__ tidx,
+                                                         int build, Fq* __restrict__ ab_out) {
+  __shared__ IpaRound s_rp;
+  if (threadIdx.x < sizeof(IpaRound) / 4) ((u32*)&s_rp)[threadIdx.x] = ((const volatile u32*)rp)[threadIdx.x];
+  __syncthreads();
+  ipa_round_block(a, b, cg, ch, n, s_rp.m, s_rp.fold != 0, s_rp.xm, s_rp.xim, build, IpaRows{1, 1 + n, 0}, fq_const_r2(), tsc, tidx, ab_out);
+}
+// The same round for a batch of proofs of one length n, one block per proof (bp_rp_prove_batch).  Proof p owns a, b, cg, ch
+// at p * n, its L/R terms at p * 2(n + 1), its final a, b at ab_out + 2p, and the Montgomery forms of its own previous
+// challenge and inverse at xs[2p], xs[2p + 1].  Terms address the rows [gs | hs | g | h | u | ...] of the generator set, the u
+// terms with c * x (umul = x R^2): the proof's u_new = x u is not a row.
+__global__ void __launch_bounds__(256) k_ipa_round_batch(Fq* __restrict__ a, Fq* __restrict__ b, Fq* __restrict__ cg, Fq* __restrict__ ch,
+                                                         u32 n, u32 m, int fold, const Fq* __restrict__ xs, int build, Fq umul,
+                                                         Fq* __restrict__ tsc, u32* __restrict__ tidx, Fq* __restrict__ ab_out) {
+  const size_t p = blockIdx.x;
+  const Fq xm = fold ? ld_fq(xs + 2 * p) : fq_zero(), xim = fold ? ld_fq(xs + 2 * p + 1) : fq_zero();
+  ipa_round_block(a + p * n, b + p * n, cg + p * n, ch + p * n, n, m, fold != 0, xm, xim, build, IpaRows{0, n, 2 * n + 2}, umul,
+                  tsc + p * 2 * (n + 1), tidx + p * 2 * (n + 1), ab_out + 2 * p);
 }
 __global__ void __launch_bounds__(128) k_to_mont(Fq* __restrict__ v, u32 n) {
   u32 t = blockIdx.x * blockDim.x + threadIdx.x;

@@ -135,9 +135,23 @@ inline bool decimal_to_fq(const uint8_t* s, size_t n, Fq* out) {
   return true;
 }
 
+// base64.b64encode (RFC 4648, with padding): the transcript's seed slot and its points
+inline std::string b64_encode(const uint8_t* raw, size_t n) {
+  static const char* A = "ABCDEFGHIJKLMNOPQRSTUVWXYZabcdefghijklmnopqrstuvwxyz0123456789+/";
+  std::string o;
+  o.reserve((n + 2) / 3 * 4);
+  for (size_t i = 0; i < n; i += 3) {
+    uint32_t v = (uint32_t)raw[i] << 16 | (i + 1 < n ? (uint32_t)raw[i + 1] << 8 : 0) | (i + 2 < n ? raw[i + 2] : 0);
+    o += A[(v >> 18) & 63];
+    o += A[(v >> 12) & 63];
+    o += i + 1 < n ? A[(v >> 6) & 63] : '=';
+    o += i + 2 < n ? A[v & 63] : '=';
+  }
+  return o;
+}
+
 // point_to_b64: utils.py:100-111.  pt = 64-byte little-endian affine, identity = zeros.
 inline std::string point_to_b64(const uint8_t pt[64]) {
-  static const char* A = "ABCDEFGHIJKLMNOPQRSTUVWXYZabcdefghijklmnopqrstuvwxyz0123456789+/";
   uint8_t raw[33];
   size_t n;
   bool ident = true;
@@ -148,15 +162,7 @@ inline std::string point_to_b64(const uint8_t pt[64]) {
     for (int i = 0; i < 32; i++) raw[1 + i] = pt[31 - i];  // x big-endian
     n = 33;
   }
-  std::string o;
-  for (size_t i = 0; i < n; i += 3) {
-    uint32_t v = (uint32_t)raw[i] << 16 | (i + 1 < n ? (uint32_t)raw[i + 1] << 8 : 0) | (i + 2 < n ? raw[i + 2] : 0);
-    o += A[(v >> 18) & 63];
-    o += A[(v >> 12) & 63];
-    o += i + 1 < n ? A[(v >> 6) & 63] : '=';
-    o += i + 2 < n ? A[v & 63] : '=';
-  }
-  return o;
+  return b64_encode(raw, n);
 }
 
 // ---- allocation-free forms for the batch verifier's per-proof transcript checks ------------------------------

@@ -1,6 +1,7 @@
 """Batch verification of independent single-value range proofs over one generator set
 (BASELINE config 5).  Not an API of the reference -- it is the data-parallel form of calling
 `RangeVerifier(V_i, g, h, gs, hs, u, proof_i).verify()` for every i, with the same decisions.
+The batch prover at the end is the same for `NIRangeProver` / `AggregNIRangeProver(...).prove()`.
 
 Packing of a proof follows include/bp_gpu.h (bp_rp_verify_batch); the per-proof transcript
 checks run in C on host threads, the scalar algebra and all point equations on the GPU.
@@ -170,6 +171,15 @@ class PackedAggregBatch(PackedBatch):
         self.m = m
         if not records:
             self.stride = nat.load().bp_rp_aggreg_proof_stride(n, m)
+
+    @classmethod
+    def from_wire(cls, n, m, nproofs, records, blob, tr_off, starts):
+        """A batch already in wire form (records back to back, the C ABI's transcript blob, offsets and start indices)."""
+        self = cls.__new__(cls)
+        self.n, self.m, self.nproofs = n, m, nproofs
+        self.stride = nat.load().bp_rp_aggreg_proof_stride(n, m)
+        self.records, self.blob, self.tr_off, self.starts = records, blob, tr_off, starts
+        return self
 
     @classmethod
     def from_proofs(cls, Vs_list, proofs, n):
@@ -395,3 +405,93 @@ def verify_mixed_range_proofs_batch(items, g, h, gs, hs, u, seed=None, locate=Fa
         else:
             out.append(a == 1)
     return out
+
+
+# ---- batch prover ---------------------------------------------------------------------------------------------------------------
+def _scalar_bytes(vals, what):
+    out = []
+    for v in vals:
+        x = int(getattr(v, "x", v))
+        if not 0 <= x < 1 << 256:
+            raise ValueError("%s must lie in [0, 2^256)" % what)
+        out.append(x.to_bytes(32, "little"))
+    return b"".join(out)
+
+
+def prove_range_proofs_packed(vs_list, n, g, h, gs, hs, gammas_list, u, seeds, packed=None):
+    """-> PackedAggregBatch of AggregNIRangeProver(vs_list[p], n, g, h, gs, hs, gammas_list[p], u, secp256k1, seeds[p]).prove()
+    for every p (NIRangeProver for m = 1 values per proof), byte for byte, in the wire form the batch verifiers read: the records
+    (V_j = v_j g + gamma_j h first; for m = 1 also a valid PackedBatch) and the three transcripts of every proof, with no Python
+    objects in between (bp_rp_prove_batch).  vs_list, gammas_list: one list of m values (ModP or int) per proof, the same m for
+    every proof; seeds: one bytes seed per proof; packed = pack_generators(g, h, gs, hs, u), as for the verifiers.
+    As in the reference, the blinding factors (alpha, rho, sL, sR, tau1, tau2) derive from the seed alone: proofs that must not
+    share them need distinct seeds.  ValueError: ragged m, mismatched lengths, or n*m not a power of two <= 2048 or not len(gs)."""
+    nproofs = len(vs_list)
+    if len(gammas_list) != nproofs or len(seeds) != nproofs:
+        raise ValueError("vs_list, gammas_list and seeds must have one entry per proof")
+    m = len(vs_list[0]) if nproofs else 1
+    if any(len(vs) != m for vs in vs_list) or any(len(gm) != m for gm in gammas_list):
+        raise ValueError("every proof of a batch aggregates the same number of values, with one gamma each")
+    N = n * m
+    if n < 1 or m < 1 or N & (N - 1) or N > 2048:
+        raise ValueError("n * m must be a power of two <= 2048")
+    if nproofs == 0:
+        return PackedAggregBatch(n, m, [], [], [])
+    gs_b, hs_b, g_b, h_b, u_b = packed if packed is not None else pack_generators(g, h, gs, hs, u)
+    if len(gs_b) != 64 * N or len(hs_b) != 64 * N:
+        raise ValueError("gs and hs must hold n * m = %d points each" % N)
+    values = _scalar_bytes([v for vs in vs_list for v in vs], "values")
+    gammas = _scalar_bytes([gm for gms in gammas_list for gm in gms], "gammas")
+    seed_off = [0]
+    for sd in seeds:
+        seed_off.append(seed_off[-1] + len(sd))
+    L = N.bit_length() - 1
+    stride = nat.load().bp_rp_aggreg_proof_stride(n, m)
+    # upper bound of the transcripts: seed slot, 4 points of 45 and 3 decimals of <= 79 bytes; Protocol 1 "&x1&" and Protocol 2's
+    # start "&&x1&"; per round 2 points and a decimal
+    cap = sum(4 * ((len(sd) + 2) // 3) for sd in seeds) + nproofs * (1 + 4 * 45 + 3 * 79 + 81 + 82 + L * (2 * 45 + 79))
+    records = ctypes.create_string_buffer(nproofs * stride)
+    blob = ctypes.create_string_buffer(cap)
+    tr_len = ctypes.c_size_t(0)
+    tr_off = (ctypes.c_uint64 * (3 * nproofs + 1))()
+    starts = (ctypes.c_uint32 * nproofs)()
+    nat.check(nat.load().bp_rp_prove_batch(gs_b, hs_b, g_b, h_b, u_b, n, m, values, gammas, b"".join(seeds),
+                                           (ctypes.c_uint64 * (nproofs + 1))(*seed_off), nproofs, records, blob, cap,
+                                           ctypes.byref(tr_len), tr_off, starts))
+    return PackedAggregBatch.from_wire(n, m, nproofs, records.raw, blob.raw[:tr_len.value], tr_off, starts)
+
+
+def unpack_aggreg_proofs(batch: PackedAggregBatch):
+    """-> list[Proof] of a packed batch (pack_aggreg_proof in reverse; the commitments V_j are not part of a Proof)."""
+    from ..innerproduct.inner_product_verifier import Proof1, Proof2
+    from ..point import Point
+    from ..utils.utils import ModP
+    from ._core import Proof
+    q, m, stride = nat.Q, batch.m, batch.stride
+    L = (batch.n * m).bit_length() - 1
+    rec, blob, offs = batch.records, batch.blob, batch.tr_off
+    sc = lambda b, o: ModP(int.from_bytes(b[o:o + 32], "little"), q)       # noqa: E731
+    out = []
+    for p in range(batch.nproofs):
+        base = p * stride
+        pt = lambda k: Point.from_bytes64(rec, base + 64 * k)               # noqa: E731  (points m, m+1, ... after the V_j)
+        A, S, T1, T2 = pt(m), pt(m + 1), pt(m + 2), pt(m + 3)
+        o = base + 64 * (m + 4)
+        taux, mu, t_hat = sc(rec, o), sc(rec, o + 32), sc(rec, o + 64)
+        u_new, P_new = Point.from_bytes64(rec, o + 96), Point.from_bytes64(rec, o + 160)
+        o += 224
+        a, b = sc(rec, o), sc(rec, o + 32)
+        o += 64
+        xs = [sc(rec, o + 32 * j) for j in range(L)]
+        Ls = [Point.from_bytes64(rec, o + 32 * L + 64 * j) for j in range(L)]
+        Rs = [Point.from_bytes64(rec, o + 96 * L + 64 * j) for j in range(L)]
+        t0, t1, t2, t3 = (offs[3 * p + k] for k in range(4))
+        p2 = Proof2(a, b, xs, Ls, Rs, blob[t2:t3], batch.starts[p])
+        out.append(Proof(taux, mu, t_hat, T1, T2, A, S, Proof1(u_new, P_new, p2, blob[t1:t2]), blob[t0:t1]))
+    return out
+
+
+def prove_range_proofs_batch(vs_list, n, g, h, gs, hs, gammas_list, u, seeds, packed=None):
+    """-> list[Proof]: the proofs of prove_range_proofs_packed (same arguments, same rules on seeds) as Python objects, equal field
+    for field to NIRangeProver / AggregNIRangeProver(...).prove()."""
+    return unpack_aggreg_proofs(prove_range_proofs_packed(vs_list, n, g, h, gs, hs, gammas_list, u, seeds, packed))
